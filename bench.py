@@ -2,6 +2,7 @@
 """bench.py -- rasterizer forward+backward throughput on the BASELINE.json workload.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200gs|reference] [--workload NAME] [--mode extended|vanilla]
+                    [--dump-outputs DIR]
 
 A "step" is one rasterizer forward+backward of one view of the named synthetic workload (default: the
 LLFF fern shape of BASELINE.json configs[0]/[1]: 100k Gaussians, 504x378, SH degree 3, the SDP-GS output
@@ -59,6 +60,9 @@ def parse():
     ap.add_argument("--no-train", action="store_true", help="skip the training-iteration measurement (`train` key)")
     ap.add_argument("--no-extras", action="store_true", help="skip the two sharded-path measurements of BASELINE.json configs[3]/[4] "
                                                                "(`render_sharded`, `stress_train` keys)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (rendered maps, radii, gradients) as "
+                         "DIR/<name>.npy in float32 (rank 0, b200gs arm; at most 64 MB in all, a fixed seeded sample beyond that)")
     return ap.parse_args()
 
 
@@ -397,14 +401,13 @@ def stress_train(args, rank, world, dev, flush):
     torch.cuda.empty_cache()
     tr = GaussianTrainer(cameras=cams, gt_images=gts, depth_mono=monos, device=dev, capacity=cap, **rp)
     tr.capture_multi(range(len(cams)))
-    steps = max(3, min(args.steps, 5))
-    ms, _ = event_loop(steps, 3, lambda i: tr.step_multi(), flush, world)
+    ms, _ = event_loop(args.steps, 3, lambda i: tr.step_multi(), flush, world)
     for sess in tr.sessions:
         assert sess.status()[1] == 0, "binning capacity overflow in stress_train"
-    ms_it = ms / steps
+    ms_it = ms / args.steps
     return dict(workload=f"stress_train: P={P}, 1920x1080, 8 views per optimizer step ({len(cams)} per rank), losses + backward + "
                          f"{'fused gradient exchange (62 floats per Gaussian) + ' if world > 1 else ''}Adam; one CUDA-graph replay per step",
-                steps_per_s=1000.0 / ms_it, views_per_s=8 * 1000.0 / ms_it, ms_per_step=ms_it, steps=steps,
+                steps_per_s=1000.0 / ms_it, views_per_s=8 * 1000.0 / ms_it, ms_per_step=ms_it, steps=args.steps,
                 exchange_bytes_per_rank=int(62 * 4 * tr.bucket.Pp * (world - 1) / world * 2) if world > 1 else 0,
                 num_rendered_mean=int(np.mean(Ls)), last_loss=tr.loss_values()[0])
 
@@ -472,6 +475,9 @@ def run_b200gs(args, rank, world, local):
             flush(); solo()
         torch.cuda.synchronize()
     ms_total, wall = event_loop(args.steps, args.warmup, step_resident, flush, world)
+    dumped = None
+    if args.dump_outputs and rank == 0:  # before anything else runs a session: the last timed step's results are still in place
+        dumped = step_outputs(sessions[(args.warmup + args.steps - 1 + rank) % nviews])
     if rank == 0:
         t_s = time.perf_counter()
         while time.perf_counter() - t_s < 0.7:  # a few more samples under the identical load
@@ -491,7 +497,7 @@ def run_b200gs(args, rank, world, local):
 
     # ---- per-stage timing (eager launches, CUDA events between stages on the launch stream)
     _lib.lib.b200gs_profile_enable(1)
-    nprof = max(5, min(args.steps, 20))
+    nprof = args.steps
     for i in range(nprof + 2):
         if i == 2:
             _lib.lib.b200gs_profile_read(None, None, 1)
@@ -614,7 +620,40 @@ def run_b200gs(args, rank, world, local):
                     gpu_launches=int(launches_per_step * args.steps), gpu_launches_per_step=int(launches_per_step),
                     clocks=clocks, roofline=roofline, cpu_baseline=cpu, vanilla=vanilla, train=train, impl="b200gs",
                     collective_check=coll, wall_s=wall, **extras)
+        if dumped is not None:
+            write_outputs(args.dump_outputs, dumped)
         print(json.dumps(line))
+
+
+DUMP_LIMIT_BYTES = 64_000_000 - 64_000  # 64 MB including the .npy headers
+
+
+def step_outputs(session):
+    """Host copies (float32) of what one step of a RasterSession hands its caller: the rendered maps, the radii and the
+    gradients it wrote."""
+    s = session
+    out = dict(color=s.color, radii=s.radii)
+    if s.extended:
+        out.update(depth=s.depth, alpha=s.alpha, feature=s.feature)
+    for k, g in getattr(s, "grads", {}).items():
+        if g is not None:
+            out["grad_" + k] = g
+    torch.cuda.synchronize()
+    return {k: v.detach().cpu().numpy().astype(np.float32) for k, v in out.items()}
+
+
+def write_outputs(d, arrays, limit=DUMP_LIMIT_BYTES):
+    """DIR/<name>.npy per array.  Above `limit` bytes in all, every array is cut to the same share of its elements, taken at
+    fixed-seed indices of the flattened array (sorted; the same indices for the same shape, so two builds compare element for
+    element)."""
+    os.makedirs(d, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > limit:
+            keep = a.size * limit // total
+            a = a.reshape(-1)[np.unique(np.random.default_rng(0).integers(0, a.size, keep))]
+        np.save(os.path.join(d, name + ".npy"), a)
+    print(f"bench.py: wrote {len(arrays)} arrays of the last timed step to {d}", file=sys.stderr)
 
 
 def train_targets(wl):

@@ -17,9 +17,11 @@ machine independent).  Stored per case (npz):
 The config-1 shape (P=100k, 504x378) is stored as SHA-256 digests + summary statistics (json).
 """
 import hashlib
+import io
 import json
 import os
 import sys
+import zipfile
 
 import numpy as np
 
@@ -78,7 +80,7 @@ def main(outdir, only=None):
             conic_opacity=base["conic_opacity"], tiles_touched=base["tiles_touched"],
             num_rendered=np.int64(base["num_rendered"]), point_list=base["point_list"],
             point_list_keys=base["point_list_keys"], ranges=base["ranges"], n_contrib=base["n_contrib"],
-            final_T=base["final_T"], color=base["color"], rgb=np.asarray(base["rgb"], np.float32))
+            final_T=base["final_T"], color=base["color"])
         for k, v in base["grads"].items():
             arrays["grad_" + k] = v
         if inp["extended"]:
@@ -87,7 +89,12 @@ def main(outdir, only=None):
             for k, v in ext["grads"].items():
                 arrays["extgrad_" + k] = v
         path = os.path.join(outdir, name + ".npz")
-        np.savez_compressed(path, **arrays)
+        # an npz that np.load reads, LZMA-compressed: keeps the largest case (small_sh3) under 1 MB
+        with zipfile.ZipFile(path, "w", compression=zipfile.ZIP_LZMA) as z:
+            for k, v in arrays.items():
+                buf = io.BytesIO()
+                np.save(buf, v)
+                z.writestr(k + ".npy", buf.getvalue())
         print(name, "P", inp["means3D"].shape[0], "L", base["num_rendered"], os.path.getsize(path), "bytes")
 
     if only:

@@ -154,6 +154,30 @@ def test_reference_arm_of_the_bench_never_imports_the_product_library():
     assert out == "False"
 
 
+def test_bench_output_dump_is_whole_below_the_limit_and_a_fixed_sample_above(tmp_path):
+    """bench.py --dump-outputs: arrays are written whole while they fit the limit; above it every array is cut to the same share
+    of its elements, at the same indices on every run."""
+    import numpy as np
+    import bench
+    rng = np.random.default_rng(3)
+    arrays = dict(grad_shs=rng.normal(size=(1000, 16, 3)).astype(np.float32), radii=rng.integers(0, 9, 1000).astype(np.float32))
+    load = lambda d: {k: np.load(os.path.join(d, k + ".npy")) for k in arrays}
+    bench.write_outputs(str(tmp_path / "whole"), arrays)
+    for k, a in load(str(tmp_path / "whole")).items():
+        np.testing.assert_array_equal(a, arrays[k])
+    limit = 20_000
+    runs = []
+    for name in ("s1", "s2"):
+        bench.write_outputs(str(tmp_path / name), arrays, limit=limit)
+        runs.append(load(str(tmp_path / name)))
+    total = sum(a.nbytes for a in arrays.values())
+    assert sum(a.nbytes for a in runs[0].values()) <= limit
+    for k in arrays:
+        np.testing.assert_array_equal(runs[0][k], runs[1][k])
+        assert runs[0][k].dtype == np.float32 and runs[0][k].size > 0.8 * arrays[k].size * limit / total
+        assert np.isin(runs[0][k], arrays[k]).all()
+
+
 def test_image_workspace_holds_the_cost_history_and_the_backward_order():
     """ImageState carries, per tile, two cost words and a second launch order (persistent workspaces): the size query must
     cover them (3 extra words per tile on top of ranges, order, counters and the two per-pixel planes)."""

@@ -209,47 +209,61 @@ def test_trainer_iterations_match_autograd_pipeline():
     assert float(tr.bucket.segment("denom").sum()) > 0
 
 
+class _OracleRasterize(torch.autograd.Function):
+    """The CPU oracle (oracle/gs_oracle.c: the reference rasterizer restated in C, held to the reference's stored outputs by
+    tests/test_oracle_golden.py) as an autograd op: the colour image of one view, from SH of degree 3 or from precomputed
+    colours, and its backward."""
+
+    @staticmethod
+    def forward(ctx, means3D, shs, colors_precomp, opacities, scales, rotations, cam, bg):
+        from oracle import cpu_oracle as orc
+        n = lambda t: None if t is None else t.detach().cpu().numpy()
+        o = orc.forward(n(means3D), n(opacities), cam, bg, shs=n(shs), colors_precomp=n(colors_precomp), scales=n(scales),
+                        rotations=n(rotations), sh_degree=3 if shs is not None else 0)
+        ctx.o, ctx.has_sh = o, shs is not None
+        return torch.from_numpy(o["color"].copy()).to(means3D.device)
+
+    @staticmethod
+    def backward(ctx, g_color):
+        from oracle import cpu_oracle as orc
+        g = orc.backward(ctx.o, g_color.detach().cpu().numpy())
+        t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(g_color.device)
+        return (t(g["means3D"]), t(g["shs"]) if ctx.has_sh else None, None if ctx.has_sh else t(g["colors_precomp"]),
+                t(g["opacities"]), t(g["scales"]), t(g["rotations"]), None, None)
+
+
 @gpu
 def test_short_fit_lands_within_a_tenth_of_a_db_of_the_reference_pipeline():
     """BASELINE.json: "a full few-shot run must land within 0.1 dB PSNR of the reference".  No dataset offline, so the
     stand-in is a short fit on synthetic supervision: ground-truth images / depths are rendered from a ground-truth
-    scene by the UNMODIFIED reference CUDA rasterizer, the model starts from a perturbed copy, and the same 80
+    scene by the reference rasterizer as the CPU oracle restates it, the model starts from a perturbed copy, and the same 80
     iterations (no densification: its RNG would make the two runs incomparable) are run by (a) GaussianTrainer -- one
-    CUDA-graph replay per iteration, every kernel ours -- and (b) the reference's stock path: its rasterizer through
-    autograd + torch activations / losses / Adam (oracle/train_torch.py).  Final training PSNR must agree to 0.1 dB."""
+    CUDA-graph replay per iteration, every kernel ours -- and (b) the reference's stock path: its rasterizer (the oracle)
+    through autograd + torch activations / losses / Adam (oracle/train_torch.py).  Final training PSNR must agree to 0.1 dB."""
     from b200gs import synthetic as syn
     from b200gs.trainer import GaussianTrainer, expon_lr, DEFAULTS
-    from oracle import ref_cuda, train_torch as tt
-    if not ref_cuda.available():
-        pytest.skip("oracle/_ref not built")
+    from oracle import train_torch as tt
     dev = torch.device("cuda", 0)
     sc = syn.make_config("small")
     cams = sc.cameras
     P, H, W = sc.P, cams[0].height, cams[0].width
     t = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32)).to(dev)
-    bg = torch.zeros(3, device=dev)
-    binning_bytes = 64 << 20
+    bg = np.zeros(3, np.float32)
+    views = [t(c.viewmatrix) for c in cams]
 
-    def ref_cfgs(cam):
-        base = dict(cam=cam, view=t(cam.viewmatrix), proj=t(cam.projmatrix), campos=t(cam.campos), binning_bytes=binning_bytes)
-        return dict(base, bg=bg, D=3), dict(base, bg=bg, D=0)
-
-    cfgs = [ref_cfgs(c) for c in cams]
-
-    def ref_render(a, cfg_rgb, cfg_pack):
-        means2D = torch.zeros((P, 3), device=dev, requires_grad=True)
-        color, _ = ref_cuda.RefRasterize.apply(a["xyz"], means2D, a["shs"], None, a["opacity"], a["scaling"], a["rotation"], cfg_rgb)
-        z = a["xyz"] @ cfg_rgb["view"][:3, 2] + cfg_rgb["view"][3, 2]
+    def ref_render(a, v):
+        color = _OracleRasterize.apply(a["xyz"], a["shs"], None, a["opacity"], a["scaling"], a["rotation"], cams[v], bg)
+        z = a["xyz"] @ views[v][:3, 2] + views[v][3, 2]
         packed = torch.stack((z, torch.ones_like(z), torch.zeros_like(z)), dim=1)
-        pk, _ = ref_cuda.RefRasterize.apply(a["xyz"], means2D, None, packed, a["opacity"], a["scaling"], a["rotation"], cfg_pack)
+        pk = _OracleRasterize.apply(a["xyz"], None, packed, a["opacity"], a["scaling"], a["rotation"], cams[v], bg)
         return color, pk[0:1]
 
     # ground truth from the reference rasterizer
     gt_act = dict(xyz=t(sc.means3D), shs=t(sc.shs), opacity=t(sc.opacities), scaling=t(sc.scales), rotation=t(sc.rotations))
     gts, monos = [], []
     with torch.no_grad():
-        for c_rgb, c_pack in cfgs:
-            color, depth = ref_render(gt_act, c_rgb, c_pack)
+        for v in range(len(cams)):
+            color, depth = ref_render(gt_act, v)
             gts.append(color.clone()); monos.append(depth.clone() + 0.5)
     # perturbed start
     rng = np.random.default_rng(99)
@@ -287,14 +301,14 @@ def test_short_fit_lands_within_a_tenth_of_a_db_of_the_reference_pipeline():
         v = (it - 1) % len(cams)
         tt.set_xyz_lr(opt, expon_lr(it - 1, hp["position_lr_init"], hp["position_lr_final"], lr_delay_mult=hp["position_lr_delay_mult"],
                                     max_steps=hp["position_lr_max_steps"]))
-        color, depth = ref_render(tt.activate(leaf), *cfgs[v])
+        color, depth = ref_render(tt.activate(leaf), v)
         total, _, _, _ = tt.total_loss(color, gts[v], depth, monos[v], hp["lambda_dssim"], hp["depth_weight"])
         total.backward()
         opt.step(); opt.zero_grad(set_to_none=True)
     ref = []
     with torch.no_grad():
         for v in range(len(cams)):
-            color, _ = ref_render(tt.activate(leaf), *cfgs[v])
+            color, _ = ref_render(tt.activate(leaf), v)
             ref.append(psnr(color, gts[v]))
     start = psnr(gts[0] * 0 + 0.0, gts[0])
     print("PSNR ours", mine, "reference pipeline", ref, "(black image:", start, ")")
