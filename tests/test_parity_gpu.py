@@ -34,8 +34,12 @@ def test_vs_oracle(name):
     _require_cuda()
     inp = case_inputs(name)
     cot = case_cotangents(inp)
-    p = run_product(inp, True, cot)
-    o = run_oracle(inp, True, cot)
+    assert_matches_oracle(run_product(inp, True, cot), run_oracle(inp, True, cot))
+
+
+def assert_matches_oracle(p, o):
+    """The suite's bars against the CPU oracle: integer stages and projected geometry bit-exact, n_contrib on all but 1e-3 of
+    the pixels, maps within 1e-4, parameter gradients within 1e-3 relative."""
     assert p["num_rendered"] == o["num_rendered"]
     for k in ("radii", "tiles_touched", "rect", "point_list", "point_list_keys", "ranges"):
         np.testing.assert_array_equal(p[k], o[k], err_msg=k)
@@ -58,7 +62,12 @@ def test_vs_golden_reference_vectors(name):
     _require_cuda()
     inp = case_inputs(name)
     cot = case_cotangents(inp)
-    p = run_product(inp, True, cot)
+    assert_matches_golden(name, run_product(inp, True, cot))
+
+
+def assert_matches_golden(name, p):
+    """`p` (run_product of case `name` with its default cotangents) against the reference's stored vectors."""
+    inp = case_inputs(name)
     g = golden(name)
     assert p["num_rendered"] == int(g["num_rendered"])
     np.testing.assert_array_equal(p["radii"], g["radii"])
@@ -91,10 +100,17 @@ def test_colour_only_backward_vs_reference_vectors(name):
     (its vanilla `grad_*` vectors were made with that cotangent)."""
     _require_cuda()
     inp = case_inputs(name)
+    assert_colour_only_matches_golden(name, run_product(inp, True, colour_only_cotangents(inp)))
+
+
+def colour_only_cotangents(inp):
     cot = case_cotangents(inp)
     if inp["extended"]:  # the reference has colour only: no cotangent on the SDP-GS maps, so the gradients are comparable
         cot = (cot[0],) + tuple(np.zeros_like(c) for c in cot[1:])
-    p = run_product(inp, True, cot)
+    return cot
+
+
+def assert_colour_only_matches_golden(name, p):
     g = golden(name)
     for k in ("radii", "tiles_touched", "point_list", "point_list_keys", "ranges", "n_contrib"):
         np.testing.assert_array_equal(p[k], g[k], err_msg=k)
@@ -120,9 +136,12 @@ def _llff_inputs(view, extended=False):
 def test_full_size_digests(view):
     """config-1 shape (P=100k, 504x378): every integer stage and the image hashed against the reference run."""
     _require_cuda()
+    assert_llff_digests(view, run_product(_llff_inputs(view), backward=False))
+
+
+def assert_llff_digests(view, p):
     with open(os.path.join(GOLDEN_DIR, "llff_fern_3view.json")) as f:
         d = json.load(f)[f"view{view}"]
-    p = run_product(_llff_inputs(view), backward=False)
     sha = lambda a: hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
     assert p["num_rendered"] == d["num_rendered"]
     assert int((p["radii"] > 0).sum()) == d["visible"]
