@@ -6,11 +6,11 @@
 // stream: the caller owns the three byte workspaces and passes the stream.
 #include <atomic>
 #include <mutex>
+#include <string>
 #include <vector>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
-#include <cstring>
 #include "common.cuh"
 
 namespace {
@@ -73,18 +73,32 @@ int check_stage(const b200gs_view_t* v, cudaStream_t s, const char* what) {
 
 int train_fail(int code, const char* msg) { return fail(code, "%s", msg); }
 
-void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
-
-unsigned pdl_mask() {
-	static int v = -1;
-	if (v < 0) {
-		const char* e = getenv("B200GS_PDL");
-		v = e ? (int)(strtoul(e, nullptr, 0) & 0xFFu) : 0xFF;
-	}
-	return (unsigned)v;
+int launch_status(cudaError_t e) {
+	if (e == cudaSuccess) e = cudaGetLastError();
+	return e == cudaSuccess ? 0 : fail(B200GS_E_CUDA, "%s", cudaGetErrorString(e));
 }
 
-uint32_t higher_msb(uint32_t n) {
+void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
+
+const char* knob(Knob k) {
+	static const char* const names[KNOB_COUNT] = {"B200GS_PDL", "B200GS_BLEND_WIDE", "B200GS_BLEND_CTAS", "B200GS_SCATTER_TMA"};
+	static std::once_flag once[KNOB_COUNT];
+	static std::string value[KNOB_COUNT];
+	static bool set[KNOB_COUNT];
+	std::call_once(once[k], [k] {
+		if (const char* e = getenv(names[k])) { value[k] = e; set[k] = true; }
+	});
+	return set[k] ? value[k].c_str() : nullptr;
+}
+
+int knob_int(Knob k, int unset) {
+	const char* e = knob(k);
+	return e ? (int)strtol(e, nullptr, 0) : unset;
+}
+
+unsigned pdl_mask() { return (unsigned)knob_int(KNOB_PDL, 0xFF) & 0xFFu; }
+
+static uint32_t higher_msb(uint32_t n) {  // getHigherMsb, DGR/cuda_rasterizer/rasterizer_impl.cu:35-50
 	uint32_t msb = sizeof(n) * 4, step = msb;
 	while (step > 1) {
 		step /= 2;
@@ -92,6 +106,21 @@ uint32_t higher_msb(uint32_t n) {
 	}
 	if (n >> msb) msb++;
 	return msb;
+}
+
+TileGrid tile_grid(int W, int H) {
+	TileGrid t;
+	t.W = W;
+	t.H = H;
+	t.gx = (W + TILE_X - 1) / TILE_X;
+	t.gy = (H + TILE_Y - 1) / TILE_Y;
+	t.tiles = (size_t)t.gx * t.gy;
+	t.units = (uint32_t)(t.tiles * 8);
+	t.tile_bits = (int)higher_msb((uint32_t)t.tiles);
+	t.tile_passes = (t.tile_bits + 7) / 8;
+	t.ranges_from_emit = t.tiles <= (size_t)COUNT_TILES_MAX;
+	t.list_in_b = (t.tile_passes & 1) != 0;
+	return t;
 }
 
 // geom layout: [hdr | hist | depth look-back (4 passes) | scan state] (zeroed per forward) then the arrays
@@ -103,6 +132,7 @@ GeomState geom_from_chunk(char* base, int P) {
 	carve(p, g.hist, 8 * 256);
 	carve(p, g.lookback, (size_t)4 * sort_tiles_for(P) * 256);
 	carve(p, g.scan_state, (size_t)scan_tiles_for(P) + 1);
+	g.clean_bytes = align_up((size_t)(p - base), 256);
 	carve(p, g.depths, n);
 	carve(p, g.rect, n);
 	carve(p, g.rec, 4 * n);
@@ -115,56 +145,57 @@ GeomState geom_from_chunk(char* base, int P) {
 	return g;
 }
 
-static size_t geom_zero_len(int P) {
-	GeomState g = geom_from_chunk(nullptr, P);
-	return align_up(reinterpret_cast<size_t>(g.scan_state) + sizeof(unsigned long long) * ((size_t)scan_tiles_for(P) + 1), 256);
-}
-
-ImageState image_from_chunk(char* base, int W, int H) {
+ImageState image_from_chunk(char* base, const TileGrid& t) {
 	ImageState s;
 	char* p = base;
-	const size_t N = (size_t)W * H, tiles = (size_t)((W + TILE_X - 1) / TILE_X) * ((H + TILE_Y - 1) / TILE_Y);
+	const size_t N = (size_t)t.W * t.H, tiles = t.tiles;
 	carve(p, s.ranges, tiles ? tiles : 1);
 	carve(p, s.tile_order, tiles ? tiles : 1);
 	carve(p, s.final_T, N ? N : 1);
 	carve(p, s.n_contrib, N ? N : 1);
-	carve(p, s.tile_count, (tiles ? tiles : 1) * (size_t)tile_count_stride());
+	carve(p, s.tile_count, (tiles ? tiles : 1) * (size_t)COUNT_STRIDE);
 	carve(p, s.tile_cost, 2 * (tiles ? tiles : 1));
 	carve(p, s.tile_order_bwd, tiles ? tiles : 1);
 	s.bytes = align_up((size_t)(p - base), 256) + 256;
 	return s;
 }
 
-BinningState binning_from_chunk(char* base, int W, int H, int64_t capacity) {
+BinningState binning_from_chunk(char* base, const TileGrid& t, int64_t capacity) {
 	BinningState b;
 	char* p = base;
 	const size_t n = (size_t)(capacity > 0 ? capacity : 1);
-	const size_t tiles = (size_t)((W + TILE_X - 1) / TILE_X) * ((H + TILE_Y - 1) / TILE_Y);
-	b.surv_words = n / 32 + tiles + 2;
+	b.surv_words = n / 32 + t.tiles + 2;
 	carve(p, b.lookback, (size_t)4 * sort_tiles_for(capacity) * 256);  // up to 4 tile passes (bit <= 32)
 	carve(p, b.surv_bits, 8 * b.surv_words);
 	carve(p, b.key_a, n);
 	carve(p, b.key_b, n);
 	carve(p, b.val_a, n);
 	carve(p, b.val_b, n);
-	b.sorted_keys = b.key_a;
-	b.sorted_vals = b.val_a;
+	b.sorted_keys = t.list_in_b ? b.key_b : b.key_a;  // where the tile sort's last pass leaves the list
+	b.sorted_vals = t.list_in_b ? b.val_b : b.val_a;
 	b.bytes = align_up((size_t)(p - base), 256) + 256;
 	return b;
 }
 
-static void resolve_sorted(const b200gs_view_t* v, BinningState& bs) {
-	const uint32_t gx = (v->width + TILE_X - 1) / TILE_X, gy = (v->height + TILE_Y - 1) / TILE_Y;
-	const int passes = ((int)higher_msb(gx * gy) + 7) / 8;
-	bs.sorted_keys = (passes & 1) ? bs.key_b : bs.key_a;
-	bs.sorted_vals = (passes & 1) ? bs.val_b : bs.val_a;
+static RasterPlan plan_call(const b200gs_view_t* v, int P, const b200gs_workspace_t* ws, int64_t capacity) {
+	RasterPlan pl;
+	pl.v = v;
+	pl.grid = tile_grid(v->width, v->height);
+	pl.P = P;
+	pl.capacity = capacity;
+	pl.persistent = ws->persistent != 0;
+	pl.gs = geom_from_chunk(reinterpret_cast<char*>(ws->geom), P);
+	pl.is = image_from_chunk(reinterpret_cast<char*>(ws->image), pl.grid);
+	pl.bs = binning_from_chunk(reinterpret_cast<char*>(ws->binning), pl.grid, capacity);
+	return pl;
 }
 
-static int validate(const b200gs_view_t* v, const b200gs_gaussians_t* g, const b200gs_workspace_t* ws) {
+// Checks the arguments every rasterizer call shares and plans the call (`capacity` is checked by the callers that use it).
+static int validate(RasterPlan& pl, const b200gs_view_t* v, const b200gs_gaussians_t* g, const b200gs_workspace_t* ws, int64_t capacity) {
 	if (!v || !g || !ws) return fail(B200GS_E_ARG, "null argument");
 	if (g->P < 0 || v->width <= 0 || v->height <= 0) return fail(B200GS_E_ARG, "bad sizes P=%d W=%d H=%d", g->P, v->width, v->height);
-	if (((v->width + TILE_X - 1) / TILE_X) > 65535 || ((v->height + TILE_Y - 1) / TILE_Y) > 65535)
-		return fail(B200GS_E_ARG, "image too large for 16-bit tile rects");
+	pl = plan_call(v, g->P, ws, capacity);
+	if (pl.grid.gx > 65535 || pl.grid.gy > 65535) return fail(B200GS_E_ARG, "image too large for 16-bit tile rects");
 	if (g->P > 0) {
 		if (!g->means3D || !g->opacities) return fail(B200GS_E_ARG, "means3D and opacities are required");
 		if ((g->shs == nullptr) == (g->colors_precomp == nullptr))
@@ -177,9 +208,58 @@ static int validate(const b200gs_view_t* v, const b200gs_gaussians_t* g, const b
 		if (v->sh_degree < 0 || v->sh_degree > 3) return fail(B200GS_E_ARG, "sh_degree must be 0..3");
 	}
 	if (!v->background || !v->viewmatrix || !v->projmatrix || !v->campos) return fail(B200GS_E_ARG, "view pointers are required");
-	if (!ws->geom || ws->geom_bytes < b200gs_geom_bytes(g->P)) return fail(B200GS_E_ARG, "geom workspace too small");
-	if (!ws->image || ws->image_bytes < b200gs_image_bytes(v->width, v->height)) return fail(B200GS_E_ARG, "image workspace too small");
+	if (!ws->geom || ws->geom_bytes < pl.gs.bytes) return fail(B200GS_E_ARG, "geom workspace too small");
+	if (!ws->image || ws->image_bytes < pl.is.bytes) return fail(B200GS_E_ARG, "image workspace too small");
 	return 0;
+}
+
+static int check_binning(const RasterPlan& pl, const b200gs_workspace_t* ws) {
+	if (!ws->binning || ws->binning_bytes < pl.bs.bytes) return fail(B200GS_E_ARG, "binning workspace too small");
+	return 0;
+}
+
+static int check_preprocess_args(const RasterPlan& pl, const b200gs_outputs_t* out) {
+	if (!out || (pl.P > 0 && !out->radii)) return fail(B200GS_E_ARG, "radii output is required");
+	return 0;
+}
+
+static int check_render_args(const RasterPlan& pl, const b200gs_outputs_t* out, const b200gs_workspace_t* ws) {
+	if (!out || !out->color) return fail(B200GS_E_ARG, "color output is required");
+	if (pl.v->extended && (!out->depth || !out->alpha || !out->feature)) return fail(B200GS_E_ARG, "extended outputs are required");
+	if (pl.capacity < 0) return fail(B200GS_E_ARG, "negative capacity");
+	if (pl.capacity >= (1ll << 30)) return fail(B200GS_E_ARG, "capacity exceeds 2^30 instances (30-bit look-back counters)");
+	return check_binning(pl, ws);
+}
+
+static int forward_preprocess(const RasterPlan& pl, const b200gs_outputs_t* out, const b200gs_gaussians_t* g, cudaStream_t stream) {
+	if (!pl.persistent || pl.P == 0) {  // persistent workspaces are left clean by the previous forward's blend kernel
+		StageScope t(stream, ST_MEMSET);
+		cudaMemsetAsync(pl.gs.hdr, 0, pl.gs.clean_bytes, stream);
+		if (pl.P == 0) cudaMemsetAsync(pl.is.ranges, 0, pl.grid.tiles * sizeof(uint2), stream);  // otherwise zeroed by the preprocess kernel (rasterizer_impl.cu:310)
+	}
+	if (pl.P == 0) return 0;
+	{ StageScope t(stream, ST_PREPROCESS); launch_preprocess_forward(pl, *g, out->radii, stream); }
+	if (int e = check_stage(pl.v, stream, "preprocess")) return e;
+	{ StageScope t(stream, ST_DEPTH_SORT); launch_depth_order(pl, stream); }
+	return check_stage(pl.v, stream, "depth order");
+}
+
+// chained: the previous kernel in the stream is our depth sort
+static int forward_render(const RasterPlan& pl, const b200gs_outputs_t* out, cudaStream_t stream, bool chained) {
+	const bool emitted = pl.P > 0 && pl.capacity > 0;
+	if (emitted) {
+		{ StageScope t(stream, ST_EMIT); launch_scan_emit(pl, stream, chained); }
+		if (int e = check_stage(pl.v, stream, "instance offsets / duplicate-with-keys")) return e;
+		{ StageScope t(stream, ST_TILE_SORT); launch_tile_sort(pl, stream); }
+		if (int e = check_stage(pl.v, stream, "tile sort")) return e;
+	}
+	if (pl.P > 0 && !emitted) launch_finalize_header(pl, stream);  // the status words scan_emit assigns
+	if (!emitted || !pl.grid.ranges_from_emit) {  // small tile grids: scan_emit's last CTA already built ranges + schedule
+		{ StageScope t(stream, ST_RANGES); launch_tile_ranges(pl, emitted ? pl.capacity : 0, stream); }
+		if (int e = check_stage(pl.v, stream, "tile ranges / schedule")) return e;
+	}
+	{ StageScope t(stream, ST_BLEND_FWD); launch_blend_forward(pl, *out, stream); }
+	return check_stage(pl.v, stream, "blend forward");
 }
 
 extern "C" {
@@ -213,8 +293,10 @@ void b200gs_abi_sizes(int64_t* out6) {
 }
 
 size_t b200gs_geom_bytes(int32_t P) { return geom_from_chunk(nullptr, P).bytes; }
-size_t b200gs_image_bytes(int32_t width, int32_t height) { return image_from_chunk(nullptr, width, height).bytes; }
-size_t b200gs_binning_bytes(int64_t capacity, int32_t width, int32_t height) { return binning_from_chunk(nullptr, width, height, capacity).bytes; }
+size_t b200gs_image_bytes(int32_t width, int32_t height) { return image_from_chunk(nullptr, tile_grid(width, height)).bytes; }
+size_t b200gs_binning_bytes(int64_t capacity, int32_t width, int32_t height) {
+	return binning_from_chunk(nullptr, tile_grid(width, height), capacity).bytes;
+}
 size_t b200gs_scratch_bytes(int32_t P) { return (size_t)(P > 0 ? P : 1) * GREC_FLOATS * sizeof(float); }
 
 void b200gs_geom_layout(int32_t P, int64_t* off) {
@@ -228,17 +310,13 @@ void b200gs_geom_layout(int32_t P, int64_t* off) {
 	off[6] = (int64_t)reinterpret_cast<size_t>(g.key_a);
 }
 void b200gs_image_layout(int32_t width, int32_t height, int64_t* off) {
-	ImageState s = image_from_chunk(nullptr, width, height);
+	ImageState s = image_from_chunk(nullptr, tile_grid(width, height));
 	off[0] = (int64_t)reinterpret_cast<size_t>(s.final_T);
 	off[1] = (int64_t)reinterpret_cast<size_t>(s.n_contrib);
 	off[2] = (int64_t)reinterpret_cast<size_t>(s.ranges);
 }
 void b200gs_binning_layout(int32_t width, int32_t height, int64_t capacity, int64_t* off) {
-	BinningState b = binning_from_chunk(nullptr, width, height, capacity);
-	b200gs_view_t v;
-	memset(&v, 0, sizeof(v));
-	v.width = width; v.height = height;
-	resolve_sorted(&v, b);
+	BinningState b = binning_from_chunk(nullptr, tile_grid(width, height), capacity);
 	off[0] = (int64_t)reinterpret_cast<size_t>(b.sorted_vals);
 	off[1] = (int64_t)reinterpret_cast<size_t>(b.sorted_keys);
 }
@@ -246,7 +324,7 @@ void b200gs_binning_layout(int32_t width, int32_t height, int64_t capacity, int6
 int b200gs_workspace_init(const b200gs_workspace_t* ws, int32_t P, void* scratch, void* stream_) {
 	if (!ws || !ws->geom || P < 0 || ws->geom_bytes < b200gs_geom_bytes(P)) return fail(B200GS_E_ARG, "workspace_init: bad arguments");
 	cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-	cudaError_t e = cudaMemsetAsync(ws->geom, 0, geom_zero_len(P), stream);
+	cudaError_t e = cudaMemsetAsync(ws->geom, 0, geom_from_chunk(nullptr, P).clean_bytes, stream);
 	if (e == cudaSuccess && scratch) e = cudaMemsetAsync(scratch, 0, b200gs_scratch_bytes(P), stream);
 	if (e == cudaSuccess && ws->image && ws->image_bytes) e = cudaMemsetAsync(ws->image, 0, ws->image_bytes, stream);  // no cost history yet
 	if (e != cudaSuccess) return fail(B200GS_E_CUDA, "[CUDA ERROR] workspace_init: %s", cudaGetErrorString(e));
@@ -255,28 +333,14 @@ int b200gs_workspace_init(const b200gs_workspace_t* ws, int32_t P, void* scratch
 
 int b200gs_forward_preprocess(const b200gs_view_t* v, const b200gs_gaussians_t* g, const b200gs_outputs_t* out,
                               const b200gs_workspace_t* ws, void* stream_, int64_t* num_rendered_host) {
-	if (int e = validate(v, g, ws)) return e;
-	if (!out || (g->P > 0 && !out->radii)) return fail(B200GS_E_ARG, "radii output is required");
+	RasterPlan pl;
+	if (int e = validate(pl, v, g, ws, 0)) return e;
+	if (int e = check_preprocess_args(pl, out)) return e;
 	cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-	const int P = g->P;
-	char* gbase = reinterpret_cast<char*>(ws->geom);
-	GeomState gs = geom_from_chunk(gbase, P);
-	ImageState is = image_from_chunk(reinterpret_cast<char*>(ws->image), v->width, v->height);
-	const size_t tiles = (size_t)((v->width + TILE_X - 1) / TILE_X) * ((v->height + TILE_Y - 1) / TILE_Y);
-	if (!ws->persistent || P == 0) {  // persistent workspaces are left clean by the previous forward's blend kernel
-		StageScope t(stream, ST_MEMSET);
-		cudaMemsetAsync(gbase, 0, geom_zero_len(P), stream);
-		if (P == 0) cudaMemsetAsync(is.ranges, 0, tiles * sizeof(uint2), stream);  // otherwise zeroed by the preprocess kernel (rasterizer_impl.cu:310)
-	}
-	if (P > 0) {
-		{ StageScope t(stream, ST_PREPROCESS); launch_preprocess_forward(*v, *g, out->radii, gs, is, stream); }
-		if (int e = check_stage(v, stream, "preprocess")) return e;
-		{ StageScope t(stream, ST_DEPTH_SORT); launch_depth_order(gs, P, stream); }
-		if (int e = check_stage(v, stream, "depth order")) return e;
-	}
+	if (int e = forward_preprocess(pl, out, g, stream)) return e;
 	if (num_rendered_host) {
 		unsigned long long n = 0;
-		cudaError_t e = cudaMemcpyAsync(&n, &gs.hdr->num_acc, sizeof(n), cudaMemcpyDeviceToHost, stream);
+		cudaError_t e = cudaMemcpyAsync(&n, &pl.gs.hdr->num_acc, sizeof(n), cudaMemcpyDeviceToHost, stream);
 		if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
 		if (e != cudaSuccess) return fail(B200GS_E_CUDA, "[CUDA ERROR] reading num_rendered: %s", cudaGetErrorString(e));
 		*num_rendered_host = (int64_t)n;
@@ -284,51 +348,23 @@ int b200gs_forward_preprocess(const b200gs_view_t* v, const b200gs_gaussians_t* 
 	return 0;
 }
 
-static int forward_render_impl(const b200gs_view_t* v, const b200gs_gaussians_t* g, const b200gs_outputs_t* out,
-                               const b200gs_workspace_t* ws, int64_t capacity, void* stream_, bool chained) {
-	if (int e = validate(v, g, ws)) return e;
-	if (!out || !out->color) return fail(B200GS_E_ARG, "color output is required");
-	if (v->extended && (!out->depth || !out->alpha || !out->feature)) return fail(B200GS_E_ARG, "extended outputs are required");
-	if (capacity < 0) return fail(B200GS_E_ARG, "negative capacity");
-	if (capacity >= (1ll << 30)) return fail(B200GS_E_ARG, "capacity exceeds 2^30 instances (30-bit look-back counters)");
-	if (!ws->binning || ws->binning_bytes < b200gs_binning_bytes(capacity, v->width, v->height)) return fail(B200GS_E_ARG, "binning workspace too small");
-	cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-	const int P = g->P;
-	GeomState gs = geom_from_chunk(reinterpret_cast<char*>(ws->geom), P);
-	ImageState is = image_from_chunk(reinterpret_cast<char*>(ws->image), v->width, v->height);
-	BinningState bs = binning_from_chunk(reinterpret_cast<char*>(ws->binning), v->width, v->height, capacity);
-	resolve_sorted(v, bs);
-	const size_t tiles = (size_t)((v->width + TILE_X - 1) / TILE_X) * ((v->height + TILE_Y - 1) / TILE_Y);
-	if (P > 0 && capacity > 0) {
-		{ StageScope t(stream, ST_EMIT); launch_scan_emit(*v, gs, bs, is, P, capacity, stream, chained, ws->persistent != 0); }
-		if (int e = check_stage(v, stream, "instance offsets / duplicate-with-keys")) return e;
-		{ StageScope t(stream, ST_TILE_SORT); launch_tile_sort(*v, gs, bs, capacity, stream); }
-		if (int e = check_stage(v, stream, "tile sort")) return e;
-	}
-	const bool emitted = P > 0 && capacity > 0;
-	if (P > 0 && !emitted) launch_finalize_header(gs, capacity, stream);  // the status words scan_emit assigns
-	if (!emitted || !tile_counts_path((int)tiles)) {  // small tile grids: scan_emit's last CTA already built ranges + schedule
-		{ StageScope t(stream, ST_RANGES); launch_tile_ranges(*v, gs, bs, is, emitted ? capacity : 0, stream, ws->persistent != 0); }
-		if (int e = check_stage(v, stream, "tile ranges / schedule")) return e;
-	}
-	{
-		StageScope t(stream, ST_BLEND_FWD);
-		char* gbase = reinterpret_cast<char*>(ws->geom);
-		launch_blend_forward(*v, gs, bs, is, *out, stream, reinterpret_cast<uint4*>(gbase + sizeof(GeomHeader)),
-		                     (geom_zero_len(P) - sizeof(GeomHeader)) / sizeof(uint4), ws->persistent != 0);
-	}
-	return check_stage(v, stream, "blend forward");
-}
-
 int b200gs_forward_render(const b200gs_view_t* v, const b200gs_gaussians_t* g, const b200gs_outputs_t* out,
                           const b200gs_workspace_t* ws, int64_t capacity, void* stream) {
-	return forward_render_impl(v, g, out, ws, capacity, stream, false);
+	RasterPlan pl;
+	if (int e = validate(pl, v, g, ws, capacity)) return e;
+	if (int e = check_render_args(pl, out, ws)) return e;
+	return forward_render(pl, out, reinterpret_cast<cudaStream_t>(stream), false);
 }
 
 int b200gs_forward(const b200gs_view_t* v, const b200gs_gaussians_t* g, const b200gs_outputs_t* out,
-                   const b200gs_workspace_t* ws, int64_t capacity, void* stream) {
-	if (int e = b200gs_forward_preprocess(v, g, out, ws, stream, nullptr)) return e;
-	return forward_render_impl(v, g, out, ws, capacity, stream, g->P > 0);
+                   const b200gs_workspace_t* ws, int64_t capacity, void* stream_) {
+	RasterPlan pl;
+	if (int e = validate(pl, v, g, ws, capacity)) return e;
+	if (int e = check_preprocess_args(pl, out)) return e;
+	if (int e = check_render_args(pl, out, ws)) return e;
+	cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+	if (int e = forward_preprocess(pl, out, g, stream)) return e;
+	return forward_render(pl, out, stream, pl.P > 0);
 }
 
 int b200gs_forward_status(const b200gs_workspace_t* ws, void* stream_, int64_t* num_rendered, int32_t* overflow) {
@@ -348,7 +384,8 @@ int b200gs_forward_status(const b200gs_workspace_t* ws, void* stream_, int64_t* 
 int b200gs_backward(const b200gs_view_t* v, const b200gs_gaussians_t* g, const int32_t* radii,
                     const b200gs_workspace_t* ws, int64_t capacity, const b200gs_grad_outputs_t* gout,
                     const b200gs_grads_t* grads, void* stream_) {
-	if (int e = validate(v, g, ws)) return e;
+	RasterPlan pl;
+	if (int e = validate(pl, v, g, ws, capacity)) return e;
 	if (!gout || !grads) return fail(B200GS_E_ARG, "null gradient structs");
 	const int P = g->P;
 	if (P == 0) return 0;  // rasterize_points.cu:161
@@ -360,17 +397,13 @@ int b200gs_backward(const b200gs_view_t* v, const b200gs_gaussians_t* g, const i
 		if (!g->shs || v->sh_coeffs != 16 || !g->scales || !g->rotations)
 			return fail(B200GS_E_ARG, "gradient scatter needs shs with 16 coefficients and the scales/rotations path");
 	}
-	if (!ws->binning || ws->binning_bytes < b200gs_binning_bytes(capacity, v->width, v->height)) return fail(B200GS_E_ARG, "binning workspace too small");
+	if (int e = check_binning(pl, ws)) return e;
 	cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-	GeomState gs = geom_from_chunk(reinterpret_cast<char*>(ws->geom), P);
-	ImageState is = image_from_chunk(reinterpret_cast<char*>(ws->image), v->width, v->height);
-	BinningState bs = binning_from_chunk(reinterpret_cast<char*>(ws->binning), v->width, v->height, capacity);
-	resolve_sorted(v, bs);
 	float* grec = reinterpret_cast<float*>(grads->scratch);
-	if (!ws->persistent) { StageScope t(stream, ST_MEMSET); cudaMemsetAsync(grec, 0, b200gs_scratch_bytes(P), stream); }
-	{ StageScope t(stream, ST_BLEND_BWD); launch_blend_backward(*v, gs, bs, is, *gout, grec, stream, ws->persistent != 0); }
+	if (!pl.persistent) { StageScope t(stream, ST_MEMSET); cudaMemsetAsync(grec, 0, b200gs_scratch_bytes(P), stream); }
+	{ StageScope t(stream, ST_BLEND_BWD); launch_blend_backward(pl, *gout, grec, stream); }
 	if (int e = check_stage(v, stream, "blend backward")) return e;
-	{ StageScope t(stream, ST_PREPROCESS_BWD); launch_preprocess_backward(*v, *g, radii, gs, grec, *grads, ws->persistent != 0, stream); }
+	{ StageScope t(stream, ST_PREPROCESS_BWD); launch_preprocess_backward(pl, *g, radii, grec, *grads, stream); }
 	return check_stage(v, stream, "preprocess backward");
 }
 
@@ -391,10 +424,7 @@ int b200gs_debug_sorted_keys(const b200gs_view_t* v, int32_t P, const b200gs_wor
 	if (!v || !ws || !keys_out || !ws->geom || !ws->binning) return fail(B200GS_E_ARG, "null argument");
 	if (L > capacity) return fail(B200GS_E_ARG, "L exceeds capacity");
 	cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-	GeomState gs = geom_from_chunk(reinterpret_cast<char*>(ws->geom), P);
-	BinningState bs = binning_from_chunk(reinterpret_cast<char*>(ws->binning), v->width, v->height, capacity);
-	resolve_sorted(v, bs);
-	launch_debug_keys(*v, gs, bs, keys_out, L, stream);
+	launch_debug_keys(plan_call(v, P, ws, capacity), keys_out, L, stream);
 	cudaError_t e = cudaGetLastError();
 	if (e != cudaSuccess) return fail(B200GS_E_CUDA, "[CUDA ERROR] debug keys: %s", cudaGetErrorString(e));
 	return 0;

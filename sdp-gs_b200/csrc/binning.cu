@@ -16,8 +16,6 @@
 // out by an atomic ticket so a CTA only ever waits on CTAs that already started.  The digit
 // histograms of ALL passes are produced by the kernel that writes the keys (preprocess for the
 // depth keys, scan_emit for the tile keys), not by a separate read of the keys or inside the passes.
-#include <cstddef>
-#include <cstdlib>
 #include "common.cuh"
 
 namespace {
@@ -278,8 +276,6 @@ constexpr int EMIT_ITEMS = SCAN_ITEMS;
 // line: L2 atomics on neighbouring words serialise).  The last CTA to finish turns the totals into the tile
 // ranges, the digit histograms of the tile sort and the blend schedule, so no kernel has to re-read the sorted
 // keys.  Larger tile grids keep the separate ranges kernel (a per-instance global RED costs more than it saves).
-constexpr int COUNT_TILES_MAX = 2048;
-constexpr int COUNT_STRIDE = 32;  // words between two tiles' global counters
 
 // Launch orders of the blend units (forward, backward): tile ids, heaviest first.  Weight of a tile = what its units cost the
 // last time this workspace rendered (ImageState::tile_cost, persistent workspaces) or, without history, the length of its
@@ -566,122 +562,83 @@ __global__ void finalize_header_kernel(GeomHeader* hdr, long long capacity) {
 	hdr->overflow = (L > (unsigned long long)capacity ? 1u : 0u) | __ldcg(&hdr->prefilter_violation);
 }
 
-bool tile_counts_path(int tiles) { return tiles <= COUNT_TILES_MAX; }
-
-void launch_finalize_header(GeomState& gs, int64_t capacity, cudaStream_t stream) {
-	launch_k(PDL_EMIT, finalize_header_kernel, dim3(1), dim3(1), stream, gs.hdr, (long long)capacity);
-	count_launch();
-}
-int tile_count_stride() { return COUNT_STRIDE; }
-
-// CTAs of the radix pass kernel that are resident at once (occupancy x SM count); a fused multi-pass launch must not exceed it
-static int64_t fused_capacity(int items) {
-	static int64_t cap[2] = {-1, -1};
-	const int k = items == SORT_ITEMS_SMALL ? 0 : 1;
-	if (cap[k] < 0) {
-		static int off = -1;  // B200GS_FUSED_SORT=0: separate launches per pass (A/B)
-		if (off < 0) { const char* e = getenv("B200GS_FUSED_SORT"); off = (e && atoi(e) == 0) ? 1 : 0; }
-		int dev = 0, sms = 0, per_sm = 0;
-		cudaGetDevice(&dev);
-		cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-		if (k == 0) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, onesweep_fused_kernel<SORT_ITEMS_SMALL>, SORT_THREADS, 0);
-		else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, onesweep_fused_kernel<SORT_ITEMS_LARGE>, SORT_THREADS, 0);
-		cap[k] = off ? 0 : (int64_t)per_sm * sms;
-	}
-	return cap[k];
+void launch_finalize_header(const RasterPlan& pl, cudaStream_t stream) {
+	launch(PDL_EMIT, finalize_header_kernel, dim3(1), dim3(1), 0, stream, pl.gs.hdr, (long long)pl.capacity);
 }
 
-int launch_radix_sort(uint32_t* key_a, uint32_t* key_b, uint32_t* val_a, uint32_t* val_b, int64_t n_max,
-                      const unsigned long long* n_dev, int end_bit, uint32_t* hist, uint32_t* lookback,
-                      unsigned int* tickets, unsigned int* barrier, cudaStream_t stream) {
-	if (n_max <= 0 || end_bit <= 0) return 0;
+// stable LSD radix sort of (u32 key, u32 value) pairs on key bits [0, end_bit); n is read from *n_dev (clamped to n_max) when
+// n_dev != nullptr, else n = n_max.  The result is in (key_a, val_a) after an even number of passes, else in (key_b, val_b).
+static void launch_radix_sort(uint32_t* key_a, uint32_t* key_b, uint32_t* val_a, uint32_t* val_b, int64_t n_max,
+                              const unsigned long long* n_dev, int end_bit, uint32_t* hist /*[passes][256]*/, uint32_t* lookback,
+                              unsigned int* tickets, unsigned int* barrier /*zero on entry*/, cudaStream_t stream) {
+	if (n_max <= 0 || end_bit <= 0) return;
 	const int passes = (end_bit + 7) / 8;
 	const int items = sort_items_for(n_max);
 	const int64_t tiles = sort_tiles_for(n_max);
-	if (passes > 1 && barrier != nullptr && tiles <= fused_capacity(items)) {  // every tile's CTA fits on the device at once
-		if (items == SORT_ITEMS_SMALL)
-			launch_k(PDL_SORT, onesweep_fused_kernel<SORT_ITEMS_SMALL>, dim3((unsigned)tiles), dim3(SORT_THREADS), stream,
-				key_a, key_b, val_a, val_b, n_max, n_dev, end_bit, (const uint32_t*)hist, lookback, barrier);
-		else
-			launch_k(PDL_SORT, onesweep_fused_kernel<SORT_ITEMS_LARGE>, dim3((unsigned)tiles), dim3(SORT_THREADS), stream,
-				key_a, key_b, val_a, val_b, n_max, n_dev, end_bit, (const uint32_t*)hist, lookback, barrier);
-		count_launch();
-		return passes & 1;
+	const bool small = items == SORT_ITEMS_SMALL;
+	const dim3 grid((unsigned)tiles), block(SORT_THREADS);
+	if (passes > 1 && tiles <= (int64_t)(small ? resident_ctas<onesweep_fused_kernel<SORT_ITEMS_SMALL>>(SORT_THREADS, 0)
+	                                          : resident_ctas<onesweep_fused_kernel<SORT_ITEMS_LARGE>>(SORT_THREADS, 0))) {
+		// every tile's CTA fits on the device at once: all passes in one launch
+		auto fused = small ? onesweep_fused_kernel<SORT_ITEMS_SMALL> : onesweep_fused_kernel<SORT_ITEMS_LARGE>;
+		launch(PDL_SORT, fused, grid, block, 0, stream, key_a, key_b, val_a, val_b, n_max, n_dev, end_bit, (const uint32_t*)hist, lookback, barrier);
+		return;
 	}
+	auto pass = small ? onesweep_pass_kernel<SORT_ITEMS_SMALL> : onesweep_pass_kernel<SORT_ITEMS_LARGE>;
 	uint32_t *ki = key_a, *ko = key_b, *vi = val_a, *vo = val_b;
 	for (int p = 0; p < passes; p++) {
 		const int bits = end_bit - 8 * p < 8 ? end_bit - 8 * p : 8;
 		uint32_t* lb = lookback + (size_t)p * tiles * 256;
-		if (items == SORT_ITEMS_SMALL)
-			launch_k(PDL_SORT, onesweep_pass_kernel<SORT_ITEMS_SMALL>, dim3((unsigned)tiles), dim3(SORT_THREADS), stream,
-				ki, vi, ko, vo, n_max, n_dev, 8 * p, bits, hist + 256 * p, lb, tickets + p);
-		else
-			launch_k(PDL_SORT, onesweep_pass_kernel<SORT_ITEMS_LARGE>, dim3((unsigned)tiles), dim3(SORT_THREADS), stream,
-				ki, vi, ko, vo, n_max, n_dev, 8 * p, bits, hist + 256 * p, lb, tickets + p);
-		count_launch();
+		launch(PDL_SORT, pass, grid, block, 0, stream, ki, vi, ko, vo, n_max, n_dev, 8 * p, bits, hist + 256 * p, lb, tickets + p);
 		uint32_t* t = ki; ki = ko; ko = t;
 		t = vi; vi = vo; vo = t;
 	}
-	return passes & 1;
 }
 
 // Depth order of the P Gaussians.  After this: gs.order = ids by (depth bits, id).
-void launch_depth_order(GeomState& gs, int P, cudaStream_t stream) {
-	if (P <= 0) return;
+void launch_depth_order(const RasterPlan& pl, cudaStream_t stream) {
+	const GeomState& gs = pl.gs;
 	// keys: key_a, values: order (identity), digit histograms gs.hist[0..3]: all written by preprocess; 4 passes -> result in (key_a, order)
-	unsigned int* tickets = reinterpret_cast<unsigned int*>(reinterpret_cast<char*>(gs.hdr) + offsetof(GeomHeader, sort_ticket));
-	launch_radix_sort(gs.key_a, gs.key_b, gs.order, gs.val_b, P, nullptr, 32, gs.hist, gs.lookback, tickets, &gs.hdr->sort_barrier[0], stream);
+	launch_radix_sort(gs.key_a, gs.key_b, gs.order, gs.val_b, pl.P, nullptr, 32, gs.hist, gs.lookback, gs.hdr->sort_ticket,
+	                  &gs.hdr->sort_barrier[0], stream);
 }
 
-void launch_scan_emit(const b200gs_view_t& v, GeomState& gs, BinningState& bs, ImageState& is, int P, int64_t capacity, cudaStream_t stream, bool chained, bool history) {
-	if (P <= 0) return;
-	const uint32_t gx = (v.width + TILE_X - 1) / TILE_X, gy = (v.height + TILE_Y - 1) / TILE_Y;
-	const int bit = (int)higher_msb(gx * gy);
-	const int64_t tiles_L = sort_tiles_for(capacity);
-	const int passes = (bit + 7) / 8;
-	const int threads = scan_threads_for(P);
-	const unsigned grid = (unsigned)scan_tiles_for(P);
-	const int tiles = (int)(gx * gy);
-	uint32_t* cost = history ? is.tile_cost : (uint32_t*)nullptr;
+void launch_scan_emit(const RasterPlan& pl, cudaStream_t stream, bool chained) {
+	const GeomState& gs = pl.gs;
+	const TileGrid& t = pl.grid;
+	const int threads = scan_threads_for(pl.P);
+	const dim3 grid((unsigned)scan_tiles_for(pl.P));
+	const size_t lookback_words = (size_t)t.tile_passes * sort_tiles_for(pl.capacity) * 256;
 	auto go = [&](auto kernel) {
-		launch_impl(chained ? PDL_EMIT : 0u, kernel, dim3(grid), dim3(threads), stream, (const uint32_t*)gs.order, (const ushort4*)gs.rect, P, gx, capacity, bit,
-			bs.key_a, bs.val_a, reinterpret_cast<uint32_t*>(gs.scan_state), gs.hist + 4 * 256, bs.lookback, (size_t)passes * tiles_L * 256, gs.hdr,
-			is.tile_count, tiles, is.ranges, is.tile_order, is.tile_order_bwd, cost);
+		launch(chained ? PDL_EMIT : 0u, kernel, grid, dim3(threads), 0, stream, (const uint32_t*)gs.order, (const ushort4*)gs.rect, pl.P, t.gx,
+			pl.capacity, t.tile_bits, pl.bs.key_a, pl.bs.val_a, reinterpret_cast<uint32_t*>(gs.scan_state), gs.hist + 4 * 256, pl.bs.lookback,
+			lookback_words, gs.hdr, pl.is.tile_count, (int)t.tiles, pl.is.ranges, pl.is.tile_order, pl.is.tile_order_bwd,
+			pl.persistent ? pl.is.tile_cost : (uint32_t*)nullptr);
 	};
-	const bool counts = tile_counts_path(tiles);
+	const bool counts = t.ranges_from_emit;
 	if (threads == SCAN_THREADS_SMALL) { if (counts) go(scan_emit_kernel<true, SCAN_THREADS_SMALL>); else go(scan_emit_kernel<false, SCAN_THREADS_SMALL>); }
 	else { if (counts) go(scan_emit_kernel<true, SCAN_THREADS>); else go(scan_emit_kernel<false, SCAN_THREADS>); }
-	count_launch();
 }
 
-void launch_tile_sort(const b200gs_view_t& v, GeomState& gs, BinningState& bs, int64_t capacity, cudaStream_t stream) {
-	const uint32_t gx = (v.width + TILE_X - 1) / TILE_X, gy = (v.height + TILE_Y - 1) / TILE_Y;
-	const int bit = (int)higher_msb(gx * gy);
-	const unsigned long long* n_dev = &gs.hdr->num_rendered;
-	unsigned int* tickets = reinterpret_cast<unsigned int*>(reinterpret_cast<char*>(gs.hdr) + offsetof(GeomHeader, sort_ticket)) + 4;
-	const int where = launch_radix_sort(bs.key_a, bs.key_b, bs.val_a, bs.val_b, capacity, n_dev, bit, gs.hist + 4 * 256,
-	                                    bs.lookback, tickets, &gs.hdr->sort_barrier[1], stream);
-	bs.sorted_keys = where ? bs.key_b : bs.key_a;
-	bs.sorted_vals = where ? bs.val_b : bs.val_a;
+void launch_tile_sort(const RasterPlan& pl, cudaStream_t stream) {
+	const GeomState& gs = pl.gs;
+	const BinningState& bs = pl.bs;
+	launch_radix_sort(bs.key_a, bs.key_b, bs.val_a, bs.val_b, pl.capacity, &gs.hdr->num_rendered, pl.grid.tile_bits, gs.hist + 4 * 256,
+	                  bs.lookback, gs.hdr->sort_ticket + 4, &gs.hdr->sort_barrier[1], stream);
 }
 
-void launch_tile_ranges(const b200gs_view_t& v, GeomState& gs, BinningState& bs, ImageState& is, int64_t capacity, cudaStream_t stream, bool history) {
-	const unsigned long long* n_dev = &gs.hdr->num_rendered;
-	const int tiles = ((v.width + TILE_X - 1) / TILE_X) * ((v.height + TILE_Y - 1) / TILE_Y);
-	const int64_t n_max = capacity > 0 ? capacity : 0;
+void launch_tile_ranges(const RasterPlan& pl, int64_t n_max, cudaStream_t stream) {
 	// few CTAs (grid-stride): every CTA ends with one atomic on the same counter
 	const int64_t chunks = (n_max + 1023) / 1024;  // 256 threads x 4 keys
 	const unsigned grid = (unsigned)(n_max > 0 ? (chunks < 148 * 8 ? chunks : 148 * 8) : 1);
-	unsigned int* counter = reinterpret_cast<unsigned int*>(reinterpret_cast<char*>(gs.hdr) + offsetof(GeomHeader, ranges_done));
-	launch_k(PDL_RANGES, tile_ranges_schedule_kernel, dim3(grid), dim3(256), stream, (const uint32_t*)bs.sorted_keys, n_max, n_dev, is.ranges, tiles, is.tile_order, is.tile_order_bwd,
-	         history ? is.tile_cost : (uint32_t*)nullptr, counter);
-	count_launch();
+	const ImageState& is = pl.is;
+	launch(PDL_RANGES, tile_ranges_schedule_kernel, dim3(grid), dim3(256), 0, stream, (const uint32_t*)pl.bs.sorted_keys, n_max,
+	       &pl.gs.hdr->num_rendered, is.ranges, (int)pl.grid.tiles, is.tile_order, is.tile_order_bwd,
+	       pl.persistent ? is.tile_cost : (uint32_t*)nullptr, &pl.gs.hdr->ranges_done);
 }
 
-void launch_debug_keys(const b200gs_view_t& v, GeomState& gs, BinningState& bs, uint64_t* keys_out, int64_t L,
-                       cudaStream_t stream) {
-	(void)v;
+void launch_debug_keys(const RasterPlan& pl, uint64_t* keys_out, int64_t L, cudaStream_t stream) {
 	if (L <= 0) return;
-	debug_keys_kernel<<<(unsigned)((L + 255) / 256), 256, 0, stream>>>(bs.sorted_keys, bs.sorted_vals, gs.depths, keys_out, L);
-	count_launch();
+	launch(0u, debug_keys_kernel, dim3((unsigned)((L + 255) / 256)), dim3(256), 0, stream, pl.bs.sorted_keys, pl.bs.sorted_vals, pl.gs.depths,
+	       keys_out, L);
 }

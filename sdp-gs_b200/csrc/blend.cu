@@ -708,47 +708,13 @@ __global__ void __launch_bounds__(BLEND_WARPS * 32, WIDE ? 3 : 5) blend_backward
 	tk.leave(lane, gridDim.x * BLEND_WARPS);
 }
 
-// One persistent wave: as many CTAs as fit on the device (occupancy x SM count), never more than there are units.
-template <typename K>
-unsigned persistent_cap(K kernel, size_t smem, int limit) {
-	int dev = 0, sms = 0, per_sm = 0;
-	cudaGetDevice(&dev);
-	cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-	if (smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, BLEND_WARPS * 32, smem);
-	if (per_sm < 1) per_sm = 1;
-	if (sms < 1) sms = 148;
-	if (limit > 0 && per_sm > limit) per_sm = limit;
-	return (unsigned)(per_sm * sms);
-}
-
 // CTAs per SM of the persistent grids (forward, backward).  Fewer resident warps than units lets the ticket balance the
 // SMs; more warps hide more latency.  Defaults measured on B200 (DESIGN.md); B200GS_BLEND_CTAS=f,b overrides for A/B runs.
 int ctas_per_sm(int dir) {
-	static int v[2] = {-1, -1};
-	if (v[0] < 0) {
-		v[0] = B200GS_FWD_CTAS; v[1] = B200GS_BWD_CTAS;
-		if (const char* e = getenv("B200GS_BLEND_CTAS")) {
-			int a = 0, b = 0;
-			if (sscanf(e, "%d,%d", &a, &b) == 2) { v[0] = a; v[1] = b; }
-		}
-	}
-	return v[dir];
-}
-
-template <typename... KArgs, typename... Args>
-cudaError_t launch_blend(unsigned site, void (*kernel)(KArgs...), unsigned grid, size_t smem, cudaStream_t stream, Args&&... args) {
-	cudaLaunchConfig_t cfg = {};
-	cfg.gridDim = dim3(grid);
-	cfg.blockDim = dim3(BLEND_WARPS * 32);
-	cfg.dynamicSmemBytes = smem;
-	cfg.stream = stream;
-	cudaLaunchAttribute attr[1];
-	attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-	attr[0].val.programmaticStreamSerializationAllowed = 1;
-	cfg.attrs = attr;
-	cfg.numAttrs = (site & pdl_mask()) ? 1 : 0;
-	return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+	int a = 0, b = 0;
+	if (const char* e = knob(KNOB_BLEND_CTAS))
+		if (sscanf(e, "%d,%d", &a, &b) == 2) return dir ? b : a;
+	return dir ? B200GS_BWD_CTAS : B200GS_FWD_CTAS;
 }
 
 }  // namespace
@@ -764,43 +730,47 @@ extern "C" int b200gs_debug_blend_trace(uint32_t* host_out, int dir) {
 
 namespace {
 bool use_wide(unsigned units) {
-	static int forced = -2;
-	if (forced == -2) { const char* e = getenv("B200GS_BLEND_WIDE"); forced = e ? atoi(e) : -1; }  // 0 / 1: A/B runs
+	const int forced = knob_int(KNOB_BLEND_WIDE, -1);  // 0 / 1: A/B runs
 	return forced >= 0 ? forced != 0 : units <= WIDE_MAX_UNITS;
 }
+// One persistent wave: as many CTAs as fit on the device, never more than there are units.
 template <bool EXT, bool WIDE>
-void forward_variant(const b200gs_view_t& v, GeomState& gs, BinningState& bs, ImageState& is, const b200gs_outputs_t& out, cudaStream_t stream,
-                     uint4* clean_words, size_t clean_count, uint32_t* cost, int gx, unsigned units) {
-	static unsigned cap = 0;
+void forward_variant(const RasterPlan& pl, const b200gs_outputs_t& out, cudaStream_t stream, unsigned units) {
+	const b200gs_view_t& v = *pl.v;
+	const GeomState& gs = pl.gs;
+	const ImageState& is = pl.is;
 	constexpr size_t smem = BLEND_WARPS * sizeof(FwdSmem<EXT>);
-	if (!cap) cap = persistent_cap(blend_forward_kernel<EXT, WIDE>, smem, ctas_per_sm(0));
+	const unsigned cap = resident_ctas<blend_forward_kernel<EXT, WIDE>>(BLEND_WARPS * 32, smem, ctas_per_sm(0));
 	const unsigned want = (units + BLEND_WARPS - 1) / BLEND_WARPS;
-	launch_blend(PDL_BLEND_FWD, blend_forward_kernel<EXT, WIDE>, want < cap ? want : cap, smem, stream, (const uint2*)is.ranges,
-		(const uint32_t*)is.tile_order, (const uint32_t*)bs.sorted_vals, (const float4*)gs.rec,
-		v.width, v.height, gx, units, gs.hdr, clean_words, clean_count, bs.surv_bits, bs.surv_words, cost, v.background, is.final_T, is.n_contrib,
+	uint4* clean_words = reinterpret_cast<uint4*>(gs.hdr + 1);  // the geom clean region past the header
+	const size_t clean_count = (gs.clean_bytes - sizeof(GeomHeader)) / sizeof(uint4);
+	launch(PDL_BLEND_FWD, blend_forward_kernel<EXT, WIDE>, dim3(want < cap ? want : cap), dim3(BLEND_WARPS * 32), smem, stream,
+		(const uint2*)is.ranges, (const uint32_t*)is.tile_order, (const uint32_t*)pl.bs.sorted_vals, (const float4*)gs.rec,
+		v.width, v.height, (int)pl.grid.gx, units, gs.hdr, clean_words, clean_count, pl.bs.surv_bits, pl.bs.surv_words,
+		pl.persistent ? is.tile_cost : (uint32_t*)nullptr, v.background, is.final_T, is.n_contrib,
 		out.color, EXT ? out.depth : (float*)nullptr, EXT ? out.alpha : (float*)nullptr, EXT ? out.feature : (float*)nullptr);
 }
 template <bool EXT, bool WIDE>
-void backward_variant(const b200gs_view_t& v, GeomState& gs, BinningState& bs, ImageState& is, const b200gs_grad_outputs_t& gout, float* grec,
-                      cudaStream_t stream, uint32_t* cost, int gx, unsigned units) {
-	static unsigned cap = 0;
+void backward_variant(const RasterPlan& pl, const b200gs_grad_outputs_t& gout, float* grec, cudaStream_t stream) {
+	const b200gs_view_t& v = *pl.v;
+	const GeomState& gs = pl.gs;
+	const ImageState& is = pl.is;
+	const unsigned units = pl.grid.units;
 	constexpr size_t smem = BLEND_WARPS * sizeof(BwdSmem<EXT>);
-	if (!cap) cap = persistent_cap(blend_backward_kernel<EXT, WIDE>, smem, ctas_per_sm(1));
+	const unsigned cap = resident_ctas<blend_backward_kernel<EXT, WIDE>>(BLEND_WARPS * 32, smem, ctas_per_sm(1));
 	const unsigned want = (units + BLEND_WARPS - 1) / BLEND_WARPS;
 	// first kernel of the backward chain: its predecessor is a memset / the caller's loss kernels, so no programmatic launch
-	launch_blend(0u, blend_backward_kernel<EXT, WIDE>, want < cap ? want : cap, smem, stream, (const uint2*)is.ranges,
-		(const uint32_t*)is.tile_order_bwd, (const uint32_t*)bs.sorted_vals, (const float4*)gs.rec,
-		v.width, v.height, gx, units, &gs.hdr->blend_ticket[1], &gs.hdr->blend_exit[1], (const uint32_t*)bs.surv_bits, bs.surv_words, cost, v.background,
-		(const float*)is.final_T, (const uint32_t*)is.n_contrib, gout.dL_dcolor, EXT ? gout.dL_ddepth : (const float*)nullptr,
+	launch(0u, blend_backward_kernel<EXT, WIDE>, dim3(want < cap ? want : cap), dim3(BLEND_WARPS * 32), smem, stream,
+		(const uint2*)is.ranges, (const uint32_t*)is.tile_order_bwd, (const uint32_t*)pl.bs.sorted_vals, (const float4*)gs.rec,
+		v.width, v.height, (int)pl.grid.gx, units, &gs.hdr->blend_ticket[1], &gs.hdr->blend_exit[1], (const uint32_t*)pl.bs.surv_bits,
+		pl.bs.surv_words, pl.persistent ? is.tile_cost : (uint32_t*)nullptr, v.background, (const float*)is.final_T,
+		(const uint32_t*)is.n_contrib, gout.dL_dcolor, EXT ? gout.dL_ddepth : (const float*)nullptr,
 		EXT ? gout.dL_dalpha : (const float*)nullptr, EXT ? gout.dL_dfeature : (const float*)nullptr, grec);
 }
 }  // namespace
 
-void launch_blend_forward(const b200gs_view_t& v, GeomState& gs, BinningState& bs, ImageState& is,
-                          const b200gs_outputs_t& out, cudaStream_t stream, uint4* clean_words, size_t clean_count, bool history) {
-	uint32_t* cost = history ? is.tile_cost : nullptr;
-	const int gx = (v.width + TILE_X - 1) / TILE_X, gy = (v.height + TILE_Y - 1) / TILE_Y;
-	unsigned units = (unsigned)(gx * gy * 8);
+void launch_blend_forward(const RasterPlan& pl, const b200gs_outputs_t& out, cudaStream_t stream) {
+	unsigned units = pl.grid.units;
 	const bool wide = use_wide(units);
 #ifdef B200GS_BLEND_TRACE
 	if (const char* e = getenv("B200GS_BLEND_UNIT_RANGE")) {
@@ -808,28 +778,22 @@ void launch_blend_forward(const b200gs_view_t& v, GeomState& gs, BinningState& b
 		if (sscanf(e, "%u,%u", &lo, &hi) == 2) { cudaMemcpyToSymbol(g_unit_lo, &lo, 4); if (hi < units) units = hi; }
 	}
 #endif
-	if (v.extended) {
-		if (wide) forward_variant<true, true>(v, gs, bs, is, out, stream, clean_words, clean_count, cost, gx, units);
-		else forward_variant<true, false>(v, gs, bs, is, out, stream, clean_words, clean_count, cost, gx, units);
+	if (pl.v->extended) {
+		if (wide) forward_variant<true, true>(pl, out, stream, units);
+		else forward_variant<true, false>(pl, out, stream, units);
 	} else {
-		if (wide) forward_variant<false, true>(v, gs, bs, is, out, stream, clean_words, clean_count, cost, gx, units);
-		else forward_variant<false, false>(v, gs, bs, is, out, stream, clean_words, clean_count, cost, gx, units);
+		if (wide) forward_variant<false, true>(pl, out, stream, units);
+		else forward_variant<false, false>(pl, out, stream, units);
 	}
-	count_launch();
 }
 
-void launch_blend_backward(const b200gs_view_t& v, GeomState& gs, BinningState& bs, ImageState& is,
-                           const b200gs_grad_outputs_t& gout, float* grec, cudaStream_t stream, bool history) {
-	uint32_t* cost = history ? is.tile_cost : nullptr;
-	const int gx = (v.width + TILE_X - 1) / TILE_X, gy = (v.height + TILE_Y - 1) / TILE_Y;
-	const unsigned units = (unsigned)(gx * gy * 8);
-	const bool wide = use_wide(units);
-	if (v.extended) {
-		if (wide) backward_variant<true, true>(v, gs, bs, is, gout, grec, stream, cost, gx, units);
-		else backward_variant<true, false>(v, gs, bs, is, gout, grec, stream, cost, gx, units);
+void launch_blend_backward(const RasterPlan& pl, const b200gs_grad_outputs_t& gout, float* grec, cudaStream_t stream) {
+	const bool wide = use_wide(pl.grid.units);
+	if (pl.v->extended) {
+		if (wide) backward_variant<true, true>(pl, gout, grec, stream);
+		else backward_variant<true, false>(pl, gout, grec, stream);
 	} else {
-		if (wide) backward_variant<false, true>(v, gs, bs, is, gout, grec, stream, cost, gx, units);
-		else backward_variant<false, false>(v, gs, bs, is, gout, grec, stream, cost, gx, units);
+		if (wide) backward_variant<false, true>(pl, gout, grec, stream);
+		else backward_variant<false, false>(pl, gout, grec, stream);
 	}
-	count_launch();
 }

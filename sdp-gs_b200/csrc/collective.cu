@@ -4,7 +4,7 @@
 // = 8n bytes over NVLink/NVSwitch for n floats, against 2 * (world-1)/world * 4n for a ring: the same wire traffic,
 // but one kernel, two block-level barriers and no intermediate buffers.  With an NVLS multicast mapping the switch
 // performs the reduction (multimem.ld_reduce) and the broadcast (multimem.st): 4n/world read + 4n/world written per rank.
-#include <cstdlib>
+#include <type_traits>
 #include "common.cuh"
 #include "../../include/b200gs_collective.h"
 
@@ -12,7 +12,8 @@ int train_fail(int code, const char* msg);  // api.cu
 
 namespace {
 
-constexpr int AR_BLOCKS = 256;   // maximum grid (sizes the flag array); the launch uses ar_blocks()
+constexpr int AR_BLOCKS = 256;   // maximum grid (sizes the flag array); the launch uses AR_GRID
+constexpr int AR_GRID = 64;      // measured flat between 16 and 128 blocks (the wire is the bound), slower at 256
 // float4 per thread and step = 16 / world: ~16 NVLink requests per thread in flight cover the remote-load latency
 constexpr int AR_THREADS = 512;
 constexpr int AR_MAX_WORLD = 8;
@@ -160,14 +161,13 @@ __global__ void __launch_bounds__(AR_THREADS) gather_reduce_kernel(void* const* 
 	if (threadIdx.x == 0) *epoch_word(s_flags, rank) = epoch;
 }
 
-int ar_blocks() {
-	static int v = -1;
-	if (v < 0) {
-		const char* e = getenv("B200GS_AR_BLOCKS");
-		v = e ? atoi(e) : 64;  // measured flat between 16 and 128 blocks (the wire is the bound), slower at 256
-		if (v < 1 || v > AR_BLOCKS) v = 64;
+// Launches f(std::integral_constant<int, WORLD>) for WORLD = world, 2 <= world <= AR_MAX_WORLD.
+template <int WORLD = 2, typename F>
+cudaError_t launch_for_world(int world, F&& f) {
+	if constexpr (WORLD < AR_MAX_WORLD) {
+		if (world > WORLD) return launch_for_world<WORLD + 1>(world, f);
 	}
-	return v;
+	return f(std::integral_constant<int, WORLD>{});
 }
 
 }  // namespace
@@ -184,23 +184,12 @@ int b200gs_allreduce_sum_f32(void* const* buffers_dev, void* const* flags_dev, v
 	if (world == 1 || n_floats == 0) return 0;
 	cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
 	const int64_t n4 = n_floats / 4, off4 = offset_floats / 4;
-	if (multicast_ptr) {
-		allreduce_multimem_kernel<<<ar_blocks(), AR_THREADS, 0, stream>>>(flags_dev, reinterpret_cast<float4*>(multicast_ptr), off4, n4, rank, world);
-	} else {
-		switch (world) {
-		case 2: allreduce_p2p_kernel<2><<<ar_blocks(), AR_THREADS, 0, stream>>>(buffers_dev, flags_dev, off4, n4, rank); break;
-		case 3: allreduce_p2p_kernel<3><<<ar_blocks(), AR_THREADS, 0, stream>>>(buffers_dev, flags_dev, off4, n4, rank); break;
-		case 4: allreduce_p2p_kernel<4><<<ar_blocks(), AR_THREADS, 0, stream>>>(buffers_dev, flags_dev, off4, n4, rank); break;
-		case 5: allreduce_p2p_kernel<5><<<ar_blocks(), AR_THREADS, 0, stream>>>(buffers_dev, flags_dev, off4, n4, rank); break;
-		case 6: allreduce_p2p_kernel<6><<<ar_blocks(), AR_THREADS, 0, stream>>>(buffers_dev, flags_dev, off4, n4, rank); break;
-		case 7: allreduce_p2p_kernel<7><<<ar_blocks(), AR_THREADS, 0, stream>>>(buffers_dev, flags_dev, off4, n4, rank); break;
-		default: allreduce_p2p_kernel<8><<<ar_blocks(), AR_THREADS, 0, stream>>>(buffers_dev, flags_dev, off4, n4, rank); break;
-		}
-	}
-	count_launch();
-	cudaError_t e = cudaGetLastError();
-	if (e != cudaSuccess) return train_fail(B200GS_E_CUDA, cudaGetErrorString(e));
-	return 0;
+	if (multicast_ptr)
+		return launch_status(launch(0u, allreduce_multimem_kernel, dim3(AR_GRID), dim3(AR_THREADS), 0, stream, flags_dev,
+		                            reinterpret_cast<float4*>(multicast_ptr), off4, n4, rank, world));
+	return launch_status(launch_for_world(world, [&](auto w) {
+		return launch(0u, allreduce_p2p_kernel<decltype(w)::value>, dim3(AR_GRID), dim3(AR_THREADS), 0, stream, buffers_dev, flags_dev, off4, n4, rank);
+	}));
 }
 
 int b200gs_gather_reduce_f32(void* const* staging_dev, void* const* out_dev, void* const* flags_dev, int64_t shard_rows,
@@ -209,20 +198,10 @@ int b200gs_gather_reduce_f32(void* const* staging_dev, void* const* out_dev, voi
 	    (shard_rows & 127))
 		return train_fail(B200GS_E_ARG, "gather_reduce_f32: bad arguments (2 <= world <= 8, shard_rows a positive multiple of 128)");
 	cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-	cudaError_t e;
-	switch (world) {
-	case 2: e = launch_impl(chained ? PDL_TRAIN : 0u, gather_reduce_kernel<2>, dim3(ar_blocks()), dim3(AR_THREADS), stream, staging_dev, out_dev, flags_dev, shard_rows, rank); break;
-	case 3: e = launch_impl(chained ? PDL_TRAIN : 0u, gather_reduce_kernel<3>, dim3(ar_blocks()), dim3(AR_THREADS), stream, staging_dev, out_dev, flags_dev, shard_rows, rank); break;
-	case 4: e = launch_impl(chained ? PDL_TRAIN : 0u, gather_reduce_kernel<4>, dim3(ar_blocks()), dim3(AR_THREADS), stream, staging_dev, out_dev, flags_dev, shard_rows, rank); break;
-	case 5: e = launch_impl(chained ? PDL_TRAIN : 0u, gather_reduce_kernel<5>, dim3(ar_blocks()), dim3(AR_THREADS), stream, staging_dev, out_dev, flags_dev, shard_rows, rank); break;
-	case 6: e = launch_impl(chained ? PDL_TRAIN : 0u, gather_reduce_kernel<6>, dim3(ar_blocks()), dim3(AR_THREADS), stream, staging_dev, out_dev, flags_dev, shard_rows, rank); break;
-	case 7: e = launch_impl(chained ? PDL_TRAIN : 0u, gather_reduce_kernel<7>, dim3(ar_blocks()), dim3(AR_THREADS), stream, staging_dev, out_dev, flags_dev, shard_rows, rank); break;
-	default: e = launch_impl(chained ? PDL_TRAIN : 0u, gather_reduce_kernel<8>, dim3(ar_blocks()), dim3(AR_THREADS), stream, staging_dev, out_dev, flags_dev, shard_rows, rank); break;
-	}
-	count_launch();
-	if (e == cudaSuccess) e = cudaGetLastError();
-	if (e != cudaSuccess) return train_fail(B200GS_E_CUDA, cudaGetErrorString(e));
-	return 0;
+	return launch_status(launch_for_world(world, [&](auto w) {
+		return launch(chained ? PDL_TRAIN : 0u, gather_reduce_kernel<decltype(w)::value>, dim3(AR_GRID), dim3(AR_THREADS), 0, stream, staging_dev,
+		              out_dev, flags_dev, shard_rows, rank);
+	}));
 }
 
 }  // extern "C"

@@ -49,6 +49,7 @@ struct GeomState {
 	uint32_t* hist;          // [8][256] global digit histograms (4 depth passes, up to 4 tile passes)
 	uint32_t* lookback;      // [tiles_P][256] onesweep look-back words, reused by every depth pass
 	unsigned long long* scan_state;  // [scan_tiles] look-back words of the offsets scan
+	size_t clean_bytes;      // [hdr .. scan_state]: zero at the start of every forward
 	size_t bytes;
 };
 
@@ -66,6 +67,10 @@ struct ImageState {
 	uint32_t* tile_order_bwd;  // [tiles] launch order of the backward's units
 	size_t bytes;
 };
+// Tile grids of at most COUNT_TILES_MAX tiles take scan_emit's TILE_COUNTS path (binning.cu): its last CTA builds the tile
+// ranges and blend orders from ImageState::tile_count, which holds one counter every COUNT_STRIDE words.
+constexpr int COUNT_TILES_MAX = 2048;
+constexpr int COUNT_STRIDE = 32;  // words between two tiles' global counters
 
 struct BinningState {
 	uint32_t* key_a;  // tile ids, ping
@@ -102,48 +107,62 @@ static inline int64_t sort_tiles_for(int64_t n) {
 static inline int scan_threads_for(int64_t n) { return n <= SCAN_SMALL_MAX ? SCAN_THREADS_SMALL : SCAN_THREADS; }
 static inline int64_t scan_tiles_for(int64_t n) { const int t = scan_threads_for(n); return (n + t - 1) / t; }
 
-GeomState geom_from_chunk(char* base, int P);
-ImageState image_from_chunk(char* base, int W, int H);
-BinningState binning_from_chunk(char* base, int W, int H, int64_t capacity);
-uint32_t higher_msb(uint32_t n);  // getHigherMsb, DGR/cuda_rasterizer/rasterizer_impl.cu:35-50
+// The 16x16 tile grid of one view and everything the stages derive from it.
+struct TileGrid {
+	int W, H;
+	uint32_t gx, gy, units;  // units: 8 blend units per tile
+	size_t tiles;
+	int tile_bits, tile_passes;  // key bits of the tile sort (getHigherMsb(tiles), rasterizer_impl.cu:35-50) and its radix passes
+	bool ranges_from_emit;       // tiles <= COUNT_TILES_MAX: scan_emit's last CTA builds the ranges and blend orders
+	bool list_in_b;              // odd pass count: the sorted list ends in BinningState::key_b / val_b
+};
+TileGrid tile_grid(int W, int H);
 
-void count_launch(int n = 1);
+GeomState geom_from_chunk(char* base, int P);
+ImageState image_from_chunk(char* base, const TileGrid& t);
+BinningState binning_from_chunk(char* base, const TileGrid& t, int64_t capacity);  // sorted_keys / sorted_vals per t.list_in_b
+
+// What one rasterizer call works on, derived once from its arguments and handed to every stage launcher.
+struct RasterPlan {
+	const b200gs_view_t* v;
+	TileGrid grid;
+	int P;
+	int64_t capacity;
+	bool persistent;  // the workspaces persist across calls: blend units ordered by (and recording) ImageState::tile_cost
+	GeomState gs;
+	ImageState is;
+	BinningState bs;
+};
 
 // ---- stage launchers (each enqueues on `stream`) ----
-void launch_preprocess_forward(const b200gs_view_t& v, const b200gs_gaussians_t& g, int32_t* radii, GeomState& gs,
-                               ImageState& is, cudaStream_t stream);
-void launch_preprocess_backward(const b200gs_view_t& v, const b200gs_gaussians_t& g, const int32_t* radii,
-                                GeomState& gs, float* grec, const b200gs_grads_t& gr, bool rezero_grec, cudaStream_t stream);
+void launch_preprocess_forward(const RasterPlan& pl, const b200gs_gaussians_t& g, int32_t* radii, cudaStream_t stream);
+void launch_preprocess_backward(const RasterPlan& pl, const b200gs_gaussians_t& g, const int32_t* radii, float* grec,
+                                const b200gs_grads_t& gr, cudaStream_t stream);
 void launch_mark_visible(int P, const float* means3D, const float* viewmatrix, uint8_t* present, cudaStream_t stream);
 
-// stable LSD radix sort of (u32 key, u32 value) pairs on key bits [0, end_bit); n is read from
-// *n_dev (clamped to n_max) when n_dev != nullptr, else n = n_max.  Returns which buffer pair
-// holds the result (0: a, 1: b).
-int launch_radix_sort(uint32_t* key_a, uint32_t* key_b, uint32_t* val_a, uint32_t* val_b, int64_t n_max,
-                      const unsigned long long* n_dev, int end_bit, uint32_t* hist /*[passes][256]*/,
-                      uint32_t* lookback, unsigned int* tickets, unsigned int* barrier /*zero on entry, or nullptr: one launch per pass*/,
-                      cudaStream_t stream);
-bool tile_counts_path(int tiles);  // scan_emit also produces tile ranges + blend schedule (small tile grids)
-int tile_count_stride();
-void launch_depth_order(GeomState& gs, int P, cudaStream_t stream);                     // stable sort of Gaussian ids by depth bits
-void launch_scan_emit(const b200gs_view_t& v, GeomState& gs, BinningState& bs, ImageState& is, int P, int64_t capacity, cudaStream_t stream,
-                      bool chained /* the previous kernel in the stream is our depth sort */, bool history /* order the blend units by ImageState::tile_cost */);
-void launch_tile_sort(const b200gs_view_t& v, GeomState& gs, BinningState& bs, int64_t capacity, cudaStream_t stream);
-void launch_tile_ranges(const b200gs_view_t& v, GeomState& gs, BinningState& bs, ImageState& is, int64_t capacity, cudaStream_t stream, bool history);
-void launch_debug_keys(const b200gs_view_t& v, GeomState& gs, BinningState& bs, uint64_t* keys_out, int64_t L,
-                       cudaStream_t stream);
+void launch_depth_order(const RasterPlan& pl, cudaStream_t stream);  // stable sort of Gaussian ids by depth bits
+void launch_scan_emit(const RasterPlan& pl, cudaStream_t stream, bool chained /* the previous kernel in the stream is our depth sort */);
+void launch_tile_sort(const RasterPlan& pl, cudaStream_t stream);
+void launch_tile_ranges(const RasterPlan& pl, int64_t n_max /* 0: nothing was emitted */, cudaStream_t stream);
+void launch_finalize_header(const RasterPlan& pl, cudaStream_t stream);
+void launch_debug_keys(const RasterPlan& pl, uint64_t* keys_out, int64_t L, cudaStream_t stream);
 
-void launch_blend_forward(const b200gs_view_t& v, GeomState& gs, BinningState& bs, ImageState& is,
-                          const b200gs_outputs_t& out, cudaStream_t stream, uint4* clean_words, size_t clean_count,
-                          bool history /* record the units' cost in ImageState::tile_cost */);  // also writes bs.surv_bits
-void launch_finalize_header(GeomState& gs, int64_t capacity, cudaStream_t stream);
-void launch_blend_backward(const b200gs_view_t& v, GeomState& gs, BinningState& bs, ImageState& is,
-                           const b200gs_grad_outputs_t& gout, float* grec, cudaStream_t stream, bool history);
+void launch_blend_forward(const RasterPlan& pl, const b200gs_outputs_t& out, cudaStream_t stream);  // also writes bs.surv_bits
+void launch_blend_backward(const RasterPlan& pl, const b200gs_grad_outputs_t& gout, float* grec, cudaStream_t stream);
+
+// Environment knobs, each read once, when first asked for: the value, or nullptr / `unset` when the variable is not set.
+enum Knob { KNOB_PDL, KNOB_BLEND_WIDE, KNOB_BLEND_CTAS, KNOB_SCATTER_TMA, KNOB_COUNT };
+const char* knob(Knob k);
+int knob_int(Knob k, int unset);
+
+// 0 after a successful launch (`e`, then cudaGetLastError), else B200GS_E_CUDA with the error's name as the last error
+int launch_status(cudaError_t e);
+void count_launch();
 
 // ---- device helpers ----
 #ifdef __CUDACC__
 // Programmatic dependent launch (sm_90+): every kernel of the chain is launched with
-// cudaLaunchAttributeProgrammaticStreamSerialization (launch_k below).  pdl_trigger() lets the NEXT kernel's CTAs
+// cudaLaunchAttributeProgrammaticStreamSerialization (launch() below).  pdl_trigger() lets the NEXT kernel's CTAs
 // become resident while this one is still running; pdl_wait() blocks until every earlier kernel in the stream
 // has completed and its writes are visible.  Rule used throughout: trigger first, touch only shared memory
 // and registers, then wait before the first global access.  Without the launch attribute both are no-ops.
@@ -157,12 +176,17 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 unsigned pdl_mask();  // B200GS_PDL=<bitmask of launch sites> (0 turns programmatic launches off; A/B measurements)
 enum PdlSite { PDL_SORT = 1, PDL_EMIT = 2, PDL_RANGES = 4, PDL_BLEND_FWD = 8, PDL_PRE_BWD = 16, PDL_TRAIN = 32 };
 
+// Every kernel is launched here, and counted (b200gs_launch_count).  A site enabled in pdl_mask() makes it a programmatic
+// launch: its predecessor in the stream must be one of OUR kernels, all of which execute pdl_wait.  Site 0 gives full stream
+// ordering, for the first kernel of a chain, whose predecessor is a memset / copy / foreign kernel (measured: a programmatic
+// launch behind cudaMemsetAsync may start before the memset has landed).
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_impl(unsigned site, void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t stream, Args&&... args) {
+inline cudaError_t launch(unsigned site, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args&&... args) {
+	count_launch();
 	cudaLaunchConfig_t cfg = {};
 	cfg.gridDim = grid;
 	cfg.blockDim = block;
-	cfg.dynamicSmemBytes = 0;
+	cfg.dynamicSmemBytes = smem;
 	cfg.stream = stream;
 	cudaLaunchAttribute attr[1];
 	attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -171,16 +195,24 @@ inline cudaError_t launch_impl(unsigned site, void (*kernel)(KArgs...), dim3 gri
 	cfg.numAttrs = (site & pdl_mask()) ? 1 : 0;
 	return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
-// kernel whose predecessor in the stream is one of OUR kernels (all of which execute pdl_wait): programmatic launch
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_k(unsigned site, void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t stream, Args&&... args) {
-	return launch_impl(site, kernel, grid, block, stream, static_cast<Args&&>(args)...);
-}
-// first kernel of a chain: its predecessor is a memset / copy / foreign kernel, so it is launched with full stream
-// ordering (measured: a programmatic launch behind cudaMemsetAsync may start before the memset has landed)
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_k_first(void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t stream, Args&&... args) {
-	return launch_impl(0u, kernel, grid, block, stream, static_cast<Args&&>(args)...);
+
+// CTAs of KERNEL resident on the device at once (occupancy x SM count, at most per_sm_limit per SM when > 0), computed once
+// per kernel.  Dynamic shared memory above 48 KB is opted into first.
+template <auto KERNEL>
+unsigned resident_ctas(int block, size_t smem, int per_sm_limit = 0) {
+	static unsigned ctas = 0;
+	if (!ctas) {
+		int dev = 0, sms = 0, per_sm = 0;
+		cudaGetDevice(&dev);
+		cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+		if (smem > 48 * 1024) cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+		cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, KERNEL, block, smem);
+		if (per_sm < 1) per_sm = 1;
+		if (sms < 1) sms = 148;
+		if (per_sm_limit > 0 && per_sm > per_sm_limit) per_sm = per_sm_limit;
+		ctas = (unsigned)(per_sm * sms);
+	}
+	return ctas;
 }
 // a0*b0 + a1*b1 + a2*b2 with the rounding sequence the reference's sm_100a build executes
 // (FMUL, FFMA, FFMA); pinned with .rn intrinsics so neither cicc nor ptxas may re-associate.

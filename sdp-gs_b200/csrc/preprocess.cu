@@ -6,7 +6,6 @@
 // are part of the bit-exact contract, so every operation that feeds them is written with
 // round-to-nearest intrinsics in the order the reference's sm_100a build executes them (read off
 // its SASS: cicc *and* ptxas contract mul+add into fma there, e.g. det = fma(a, c, -(b*b))).
-#include <cstdlib>
 #include "common.cuh"
 #include "tma.cuh"
 
@@ -787,8 +786,9 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_backward_kernel(
 
 }  // namespace
 
-void launch_preprocess_forward(const b200gs_view_t& v, const b200gs_gaussians_t& g, int32_t* radii, GeomState& gs,
-                               ImageState& is, cudaStream_t stream) {
+void launch_preprocess_forward(const RasterPlan& pl, const b200gs_gaussians_t& g, int32_t* radii, cudaStream_t stream) {
+	const b200gs_view_t& v = *pl.v;
+	const GeomState& gs = pl.gs;
 	const int P = g.P;
 	const float focal_y = v.height / (2.0f * v.tan_fovy);  // rasterizer_impl.cu:222-223
 	const float focal_x = v.width / (2.0f * v.tan_fovx);
@@ -796,17 +796,17 @@ void launch_preprocess_forward(const b200gs_view_t& v, const b200gs_gaussians_t&
 	const int tma_ok = al16(g.means3D) && al16(g.scales) && al16(g.rotations) && al16(g.opacities) && al16(g.shs) &&
 	                   al16(g.cov3D_precomp) && al16(g.colors_precomp) && al16(g.language_feature_precomp) &&
 	                   al16(g.shs_language) && al16(g.confidence);
-	launch_k_first(preprocess_forward_kernel, dim3((P + PRE_THREADS - 1) / PRE_THREADS), dim3(PRE_THREADS), stream,
+	launch(0u, preprocess_forward_kernel, dim3((P + PRE_THREADS - 1) / PRE_THREADS), dim3(PRE_THREADS), 0, stream,
 		P, v.sh_degree, v.sh_coeffs, g.means3D, g.scales, v.scale_modifier, g.rotations, g.opacities, g.shs,
 		g.cov3D_precomp, g.colors_precomp, g.language_feature_precomp, g.shs_language, g.confidence,
 		v.viewmatrix, v.projmatrix, v.campos, v.width, v.height, v.tan_fovx, v.tan_fovy, focal_x, focal_y,
-		v.extended, v.prefiltered, radii, gs.depths, gs.rect, gs.rec, gs.clamped, gs.key_a, gs.order, gs.hist, is.ranges, is.tile_count, tile_count_stride(),
-		((v.width + TILE_X - 1) / TILE_X) * ((v.height + TILE_Y - 1) / TILE_Y), gs.hdr, tma_ok, g.live_count);
-	count_launch();
+		v.extended, v.prefiltered, radii, gs.depths, gs.rect, gs.rec, gs.clamped, gs.key_a, gs.order, gs.hist, pl.is.ranges, pl.is.tile_count,
+		COUNT_STRIDE, (int)pl.grid.tiles, gs.hdr, tma_ok, g.live_count);
 }
 
-void launch_preprocess_backward(const b200gs_view_t& v, const b200gs_gaussians_t& g, const int32_t* radii,
-                                GeomState& gs, float* grec, const b200gs_grads_t& gr, bool rezero_grec, cudaStream_t stream) {
+void launch_preprocess_backward(const RasterPlan& pl, const b200gs_gaussians_t& g, const int32_t* radii, float* grec,
+                                const b200gs_grads_t& gr, cudaStream_t stream) {
+	const b200gs_view_t& v = *pl.v;
 	const int P = g.P;
 	const float focal_y = v.height / (2.0f * v.tan_fovy);
 	const float focal_x = v.width / (2.0f * v.tan_fovx);
@@ -815,19 +815,16 @@ void launch_preprocess_backward(const b200gs_view_t& v, const b200gs_gaussians_t
 	                   al16(g.shs_language) && al16(g.confidence) && al16(grec) && al16(gr.dL_dmeans3D) && al16(gr.dL_dmeans2D) &&
 	                   al16(gr.dL_dshs) && al16(gr.dL_dcolors) && al16(gr.dL_dscales) && al16(gr.dL_dcov3D) && al16(gr.dL_dfeatures) &&
 	                   al16(gr.dL_dshs_language);
-	static int scatter_tma = -1;  // B200GS_SCATTER_TMA=0: plain stores to the peer staging blocks (A/B)
-	if (scatter_tma < 0) { const char* e = getenv("B200GS_SCATTER_TMA"); scatter_tma = e ? atoi(e) : 1; }
-	launch_k(PDL_PRE_BWD, preprocess_backward_kernel, dim3((P + PRE_THREADS - 1) / PRE_THREADS), dim3(PRE_THREADS), stream,
-		P, v.sh_degree, v.sh_coeffs, g.means3D, radii, g.shs, gs.clamped, g.scales, g.rotations, v.scale_modifier,
+	const int scatter_tma = knob_int(KNOB_SCATTER_TMA, 1);  // 0: plain stores to the peer staging blocks (A/B)
+	launch(PDL_PRE_BWD, preprocess_backward_kernel, dim3((P + PRE_THREADS - 1) / PRE_THREADS), dim3(PRE_THREADS), 0, stream,
+		P, v.sh_degree, v.sh_coeffs, g.means3D, radii, g.shs, pl.gs.clamped, g.scales, g.rotations, v.scale_modifier,
 		g.cov3D_precomp, g.language_feature_precomp, g.shs_language, g.confidence, v.viewmatrix, v.projmatrix,
-		v.campos, focal_x, focal_y, v.tan_fovx, v.tan_fovy, v.extended, reinterpret_cast<float4*>(grec), rezero_grec ? 1 : 0,
+		v.campos, focal_x, focal_y, v.tan_fovx, v.tan_fovy, v.extended, reinterpret_cast<float4*>(grec), pl.persistent ? 1 : 0,
 		gr.dL_dmeans3D, gr.dL_dmeans2D, gr.dL_dshs, gr.dL_dcolors, gr.dL_dopacities, gr.dL_dscales,
 		gr.dL_drotations, gr.dL_dcov3D, gr.dL_dfeatures, gr.dL_dshs_language, tma_ok, gr.scatter_bases,
 		(long long)gr.scatter_shard_rows, (int)gr.scatter_rank, (int)gr.accumulate, scatter_tma);
-	count_launch();
 }
 
 void launch_mark_visible(int P, const float* means3D, const float* viewmatrix, uint8_t* present, cudaStream_t stream) {
-	mark_visible_kernel<<<(P + 255) / 256, 256, 0, stream>>>(P, means3D, viewmatrix, present);
-	count_launch();
+	launch(0u, mark_visible_kernel, dim3((P + 255) / 256), dim3(256), 0, stream, P, means3D, viewmatrix, present);
 }

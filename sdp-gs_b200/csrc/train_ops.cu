@@ -466,13 +466,9 @@ int b200gs_photometric_loss(const float* image, const float* gt, int32_t width, 
 	float *mA = scratch, *mB = scratch + n, *mC = scratch + 2 * n;
 	const dim3 grid((width + LT - 1) / LT, (height + LT - 1) / LT, 3), block(LT, LT);
 	// its predecessor is the rasterizer's blend kernel (ours, executes pdl_wait), but the forward kernel starts the chain plainly
-	launch_k_first(ssim_l1_forward_kernel, grid, block, stream, image, gt, (int)width, (int)height, win, mA, mB, mC, accum, hp, loss_out);
-	launch_k(PDL_TRAIN, ssim_l1_backward_kernel, grid, block, stream, image, gt, (int)width, (int)height, win, (const float*)mA,
-	         (const float*)mB, (const float*)mC, hp, dL_dimage);
-	count_launch(2);
-	cudaError_t e = cudaGetLastError();
-	if (e != cudaSuccess) return train_fail(B200GS_E_CUDA, cudaGetErrorString(e));
-	return 0;
+	launch(0u, ssim_l1_forward_kernel, grid, block, 0, stream, image, gt, (int)width, (int)height, win, mA, mB, mC, accum, hp, loss_out);
+	return launch_status(launch(PDL_TRAIN, ssim_l1_backward_kernel, grid, block, 0, stream, image, gt, (int)width, (int)height, win,
+	                            (const float*)mA, (const float*)mB, (const float*)mC, hp, dL_dimage));
 }
 
 int b200gs_depth_pearson_loss(const float* depth, const float* depth_mono, int32_t n, const b200gs_hparams_t* hp,
@@ -487,33 +483,23 @@ int b200gs_depth_pearson_loss_pseudo(const float* depth, const float* depth_ref,
 		return train_fail(B200GS_E_ARG, "depth_pearson_loss: bad arguments");
 	cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
 	const unsigned grid = (unsigned)min((n + 255) / 256, 148 * 4);
-	launch_k(PDL_TRAIN, pearson_reduce_kernel, dim3(grid), dim3(256), stream, depth, depth_ref, (int)n, accum, hp, loss_out, weight_device, (int)single_branch);
-	launch_k(PDL_TRAIN, pearson_grad_kernel, dim3(grid), dim3(256), stream, depth, depth_ref, (int)n, (const double*)(accum + 16 * ACC_SLOTS + 2), dL_ddepth);
-	count_launch(2);
-	cudaError_t e = cudaGetLastError();
-	if (e != cudaSuccess) return train_fail(B200GS_E_CUDA, cudaGetErrorString(e));
-	return 0;
+	launch(PDL_TRAIN, pearson_reduce_kernel, dim3(grid), dim3(256), 0, stream, depth, depth_ref, (int)n, accum, hp, loss_out, weight_device,
+	       (int)single_branch);
+	return launch_status(launch(PDL_TRAIN, pearson_grad_kernel, dim3(grid), dim3(256), 0, stream, depth, depth_ref, (int)n,
+	                            (const double*)(accum + 16 * ACC_SLOTS + 2), dL_ddepth));
 }
 
 int b200gs_knn3(int32_t P, const float* xyz, float* mean_dist2, int32_t* indices, void* stream_) {
 	if (P < 0 || (P > 0 && (!xyz || !mean_dist2 || !indices))) return train_fail(B200GS_E_ARG, "knn3: bad arguments");
 	if (P < 4) return train_fail(B200GS_E_ARG, "knn3: at least 4 points are needed for 3 neighbours");
 	cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-	knn3_kernel<<<(P + KNN_THREADS - 1) / KNN_THREADS, KNN_THREADS, 0, stream>>>(P, xyz, mean_dist2, indices);
-	count_launch();
-	cudaError_t e = cudaGetLastError();
-	if (e != cudaSuccess) return train_fail(B200GS_E_CUDA, cudaGetErrorString(e));
-	return 0;
+	return launch_status(launch(0u, knn3_kernel, dim3((P + KNN_THREADS - 1) / KNN_THREADS), dim3(KNN_THREADS), 0, stream, P, xyz, mean_dist2, indices));
 }
 
 int b200gs_hparams_advance(b200gs_hparams_t* hp, float lr_init, float lr_final, float lr_delay_mult, float max_steps, void* stream_) {
 	if (!hp || max_steps <= 0.f) return train_fail(B200GS_E_ARG, "hparams_advance: bad arguments");
 	cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-	launch_k(PDL_TRAIN, hparams_advance_kernel, dim3(1), dim3(32), stream, hp, lr_init, lr_final, lr_delay_mult, max_steps);
-	count_launch();
-	cudaError_t e = cudaGetLastError();
-	if (e != cudaSuccess) return train_fail(B200GS_E_CUDA, cudaGetErrorString(e));
-	return 0;
+	return launch_status(launch(PDL_TRAIN, hparams_advance_kernel, dim3(1), dim3(32), 0, stream, hp, lr_init, lr_final, lr_delay_mult, max_steps));
 }
 
 void b200gs_train_abi_sizes(int64_t* out2) { out2[0] = sizeof(b200gs_param_state_t); out2[1] = sizeof(b200gs_hparams_t); }
@@ -534,11 +520,7 @@ int b200gs_param_step(const b200gs_param_state_t* s, const b200gs_hparams_t* hp,
 	cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
 	// its predecessor is the preprocess backward or the gather kernel (ours: both execute griddepcontrol.wait) in a training step;
 	// launched with full stream ordering when used stand-alone or behind a foreign kernel (B200GS_STEP_AFTER_FOREIGN)
-	launch_k((update && !foreign) ? PDL_TRAIN : 0u, param_step_kernel, dim3(148 * 8), dim3(256), stream, *s, hp, (int)update);
-	count_launch();
-	cudaError_t e = cudaGetLastError();
-	if (e != cudaSuccess) return train_fail(B200GS_E_CUDA, cudaGetErrorString(e));
-	return 0;
+	return launch_status(launch((update && !foreign) ? PDL_TRAIN : 0u, param_step_kernel, dim3(148 * 8), dim3(256), 0, stream, *s, hp, (int)update));
 }
 
 }  // extern "C"
