@@ -693,13 +693,19 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_backward_kernel(
 					if (k < M) { row[3 * k] = shw[k] * dRGB[0]; row[3 * k + 1] = shw[k] * dRGB[1]; row[3 * k + 2] = shw[k] * dRGB[2]; }
 				}
 			}
-		} else if (valid) {
+		} else if (valid) {  // unstaged rows are written in place; with accumulate, coefficients 16.. (no gradient) keep their sums
 			float* row = dL_dshs + (size_t)idx * M * 3;
 #pragma unroll
 			for (int k = 0; k < 16; k++) {
-				if (k < M) { row[3 * k] = shw[k] * dRGB[0]; row[3 * k + 1] = shw[k] * dRGB[1]; row[3 * k + 2] = shw[k] * dRGB[2]; }
+				if (k < M) {
+					const float g0 = shw[k] * dRGB[0], g1 = shw[k] * dRGB[1], g2 = shw[k] * dRGB[2];
+					row[3 * k] = accumulate ? __fadd_rn(row[3 * k], g0) : g0;  // fl(previous + this view), as add_local
+					row[3 * k + 1] = accumulate ? __fadd_rn(row[3 * k + 1], g1) : g1;
+					row[3 * k + 2] = accumulate ? __fadd_rn(row[3 * k + 2], g2) : g2;
+				}
 			}
-			for (int i = 48; i < 3 * M; i++) row[i] = 0.f;
+			if (!accumulate)
+				for (int i = 48; i < 3 * M; i++) row[i] = 0.f;
 		}
 	}
 	// Image-parallel training: the parameter gradients of this 128-Gaussian tile go straight into the staging buffer of
@@ -713,9 +719,15 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_backward_kernel(
 		li0 = base - o * Ps;
 		fb = reinterpret_cast<float*>(scatter_bases[o]) + (size_t)scatter_rank * Ps * 64;
 	}
+	// the caller's rotation-gradient array need not be 16-byte aligned (a float4 access there faults): scalar accesses then
+	const bool rots16 = (reinterpret_cast<uintptr_t>(dL_drots) & 15u) == 0;
 	if (valid && accumulate) {  // several views per optimizer step: add what the earlier views left in the local arrays
 		if (dL_dopac) o_op += dL_dopac[idx];
-		if (dL_drots) { const float4 t = reinterpret_cast<const float4*>(dL_drots)[idx]; o_rot.x += t.x; o_rot.y += t.y; o_rot.z += t.z; o_rot.w += t.w; }
+		if (dL_drots) {
+			const float4 t = rots16 ? reinterpret_cast<const float4*>(dL_drots)[idx]
+			                        : make_float4(dL_drots[4 * idx], dL_drots[4 * idx + 1], dL_drots[4 * idx + 2], dL_drots[4 * idx + 3]);
+			o_rot.x += t.x; o_rot.y += t.y; o_rot.z += t.z; o_rot.w += t.w;
+		}
 	}
 	if (valid) {
 		if (fb) {
@@ -723,7 +735,8 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_backward_kernel(
 			reinterpret_cast<float4*>(fb + 55 * (size_t)scatter_Ps)[li0 + li] = o_rot;
 		} else {
 			if (dL_dopac) dL_dopac[idx] = o_op;
-			if (dL_drots) reinterpret_cast<float4*>(dL_drots)[idx] = o_rot;
+			if (dL_drots && rots16) reinterpret_cast<float4*>(dL_drots)[idx] = o_rot;
+			else if (dL_drots) { float* r = dL_drots + 4 * (size_t)idx; r[0] = o_rot.x; r[1] = o_rot.y; r[2] = o_rot.z; r[3] = o_rot.w; }
 		}
 	}
 	tma_store_fence();
