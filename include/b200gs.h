@@ -10,6 +10,7 @@
  *                           bound by RasterizeGaussiansCUDA        DGR/rasterize_points.cu:35-115 (pybind: DGR/ext.cpp:16)
  *   b200gs_backward      <- CudaRasterizer::Rasterizer::backward  DGR/cuda_rasterizer/rasterizer.h:55-84,
  *                           bound by RasterizeGaussiansBackwardCUDA DGR/rasterize_points.cu:117-196 (DGR/ext.cpp:17)
+ *   b200gs_backward_camera  the same, plus gradients w.r.t. viewmatrix / projmatrix / campos (no reference counterpart)
  *   b200gs_mark_visible  <- CudaRasterizer::Rasterizer::markVisible DGR/cuda_rasterizer/rasterizer.h:24-29,
  *                           bound by markVisible                   DGR/rasterize_points.cu:198-217 (DGR/ext.cpp:18)
  *   b200gs_*_bytes       <- CudaRasterizer::required<T>()          DGR/cuda_rasterizer/rasterizer_impl.h:66-72
@@ -189,6 +190,30 @@ int b200gs_backward(const b200gs_view_t* view, const b200gs_gaussians_t* g, cons
                     const b200gs_workspace_t* ws, int64_t capacity, const b200gs_grad_outputs_t* gout,
                     const b200gs_grads_t* grads, void* stream);
 
+/* Gradients w.r.t. the camera of one view (device), for pose refinement.  Indexed like b200gs_view_t's arrays, so
+ * dL_dviewmatrix[4c+r] is the gradient of element (r,c).  Entries the rasterizer never reads are written as exact zeros:
+ * row 3 of the view matrix (3, 7, 11, 15), row 2 of the projection (2, 6, 10, 14), and campos without shs.  The 35
+ * floats are assigned on every call, whatever b200gs_grads_t.accumulate says (camera gradients are per view), and are
+ * bitwise reproducible for the same inputs.  The intrinsics (tan_fov, hence focal) get no gradient. */
+typedef struct b200gs_camera_grads {
+	float* dL_dviewmatrix;  /* device f32[16], indexed like b200gs_view_t.viewmatrix; row 3 written 0 */
+	float* dL_dprojmatrix;  /* device f32[16], indexed like projmatrix; row 2 written 0 */
+	float* dL_dcampos;      /* device f32[3]; 0 without shs */
+	void* scratch;          /* b200gs_camera_scratch_bytes(P) bytes; no initialisation, contents on return unspecified */
+} b200gs_camera_grads_t;
+
+size_t b200gs_camera_scratch_bytes(int32_t P);
+
+/* b200gs_backward plus, when `cam` != NULL, the camera gradients (one more kernel launch).  b200gs_backward is this call
+ * with cam == NULL.  With cam: every pointer in it is required, and grads->scatter_bases must be NULL (camera gradients
+ * are not combined with the image-parallel gradient scatter); either violation returns B200GS_E_ARG. */
+int b200gs_backward_camera(const b200gs_view_t* view, const b200gs_gaussians_t* g, const int32_t* radii,
+                           const b200gs_workspace_t* ws, int64_t capacity, const b200gs_grad_outputs_t* gout,
+                           const b200gs_grads_t* grads, const b200gs_camera_grads_t* cam, void* stream);
+
+/* sizeof(b200gs_camera_grads_t); b200gs_abi_sizes reports the six structs before it. */
+int64_t b200gs_camera_grads_abi_size(void);
+
 /* present: device u8[P] (bool). */
 int b200gs_mark_visible(int32_t P, const float* means3D, const float* viewmatrix, const float* projmatrix,
                         uint8_t* present, void* stream);
@@ -210,7 +235,8 @@ int b200gs_debug_sorted_keys(const b200gs_view_t* view, int32_t P, const b200gs_
 int64_t b200gs_launch_count(void);
 /* Optional per-stage timing with CUDA events on the launch stream (bench.py's roofline numbers).
  * Stages: 0 memsets, 1 preprocess fwd, 2 depth sort, 3 offsets scan, 4 duplicate-with-keys, 5 tile sort,
- * 6 tile ranges, 7 blend fwd, 8 blend bwd, 9 preprocess bwd.  profile_read synchronizes the pending events and
+ * 6 tile ranges, 7 blend fwd, 8 blend bwd, 9 preprocess bwd (with the camera-gradient reduction when asked for).
+ * profile_read synchronizes the pending events and
  * returns accumulated milliseconds / call counts per stage (arrays of 10). */
 #define B200GS_NUM_STAGES 10
 void b200gs_profile_enable(int32_t on);

@@ -61,6 +61,11 @@ class Grads(C.Structure):
                 ("scatter_world", C.c_int32), ("accumulate", C.c_int32), ("reserved_", C.c_int32)]
 
 
+class CameraGrads(C.Structure):  # b200gs_camera_grads_t
+    _fields_ = [("dL_dviewmatrix", C.c_void_p), ("dL_dprojmatrix", C.c_void_p), ("dL_dcampos", C.c_void_p),
+                ("scratch", C.c_void_p)]
+
+
 class HParams(C.Structure):  # include/b200gs_train.h: b200gs_hparams_t (64 bytes, lives in device memory)
     _fields_ = [("step", C.c_float), ("lr_xyz", C.c_float), ("lr_f_dc", C.c_float), ("lr_f_rest", C.c_float),
                 ("lr_opacity", C.c_float), ("lr_scaling", C.c_float), ("lr_rotation", C.c_float), ("lr_feature", C.c_float),
@@ -89,6 +94,7 @@ EXPORTS = [
     "b200gs_forward_status", "b200gs_backward", "b200gs_mark_visible", "b200gs_geom_layout",
     "b200gs_image_layout", "b200gs_binning_layout", "b200gs_debug_sorted_keys", "b200gs_launch_count",
     "b200gs_abi_sizes", "b200gs_profile_enable", "b200gs_profile_read",
+    "b200gs_backward_camera", "b200gs_camera_scratch_bytes", "b200gs_camera_grads_abi_size",
 ]
 
 
@@ -102,8 +108,11 @@ def _load():
         if not hasattr(lib, name):
             raise ImportError(f"{LIB_PATH} does not export {name}")
     lib.b200gs_last_error.restype = C.c_char_p
-    for f in ("b200gs_geom_bytes", "b200gs_image_bytes", "b200gs_binning_bytes", "b200gs_scratch_bytes"):
+    for f in ("b200gs_geom_bytes", "b200gs_image_bytes", "b200gs_binning_bytes", "b200gs_scratch_bytes",
+              "b200gs_camera_scratch_bytes"):
         getattr(lib, f).restype = C.c_size_t
+    lib.b200gs_camera_scratch_bytes.argtypes = [C.c_int32]
+    lib.b200gs_camera_grads_abi_size.restype = C.c_int64
     lib.b200gs_geom_bytes.argtypes = [C.c_int32]
     lib.b200gs_image_bytes.argtypes = [C.c_int32, C.c_int32]
     lib.b200gs_binning_bytes.argtypes = [C.c_int64, C.c_int32, C.c_int32]
@@ -116,6 +125,8 @@ def _load():
     lib.b200gs_forward.argtypes = [P(View), P(Gaussians), P(Outputs), P(Workspace), C.c_int64, C.c_void_p]
     lib.b200gs_forward_status.argtypes = [P(Workspace), C.c_void_p, P(C.c_int64), P(C.c_int32)]
     lib.b200gs_backward.argtypes = [P(View), P(Gaussians), C.c_void_p, P(Workspace), C.c_int64, P(GradOutputs), P(Grads), C.c_void_p]
+    lib.b200gs_backward_camera.argtypes = [P(View), P(Gaussians), C.c_void_p, P(Workspace), C.c_int64, P(GradOutputs), P(Grads),
+                                           P(CameraGrads), C.c_void_p]
     lib.b200gs_mark_visible.argtypes = [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.b200gs_geom_layout.argtypes = [C.c_int32, P(C.c_int64)]
     lib.b200gs_image_layout.argtypes = [C.c_int32, C.c_int32, P(C.c_int64)]
@@ -146,6 +157,9 @@ def _load():
     mine = [C.sizeof(t) for t in (View, Gaussians, Outputs, Workspace, GradOutputs, Grads)]
     if list(sizes) != mine:
         raise ImportError(f"ABI mismatch between {LIB_PATH} {list(sizes)} and this binding {mine}")
+    if lib.b200gs_camera_grads_abi_size() != C.sizeof(CameraGrads):
+        raise ImportError(f"ABI mismatch (camera gradients) between {LIB_PATH} {lib.b200gs_camera_grads_abi_size()} and this "
+                          f"binding {C.sizeof(CameraGrads)}")
     tsizes = (C.c_int64 * 2)()
     lib.b200gs_train_abi_sizes.argtypes = [P(C.c_int64)]
     lib.b200gs_train_abi_sizes(tsizes)

@@ -13,7 +13,7 @@ import ctypes as C
 import torch
 
 from . import _lib
-from ._lib import Gaussians, GradOutputs, Grads, Outputs, View, Workspace, check, lib
+from ._lib import CameraGrads, Gaussians, GradOutputs, Grads, Outputs, View, Workspace, check, lib
 
 # When not None: binning capacity (instances) used instead of the reference's blocking D2H read of
 # num_rendered (DGR/cuda_rasterizer/rasterizer_impl.cu:281).  See set_binning_capacity().
@@ -247,9 +247,18 @@ def _forward_impl(rs, means3D, sh, colors_precomp, opacities, scales, rotations,
     return num_rendered, capacity, color, depth, alpha, feature, radii, geom, binning, img
 
 
+def _camera_grads(flat, like):
+    """The 35 floats of b200gs_camera_grads_t as gradients with the (shape, dtype) of the viewmatrix, projmatrix and
+    campos tensors in `like`: the kernels index them like the contiguous float32 copies the forward read, i.e. in the
+    tensors' logical element order."""
+    return tuple(flat[o:o + n].view(shape).to(dtype) for (o, n), (shape, dtype) in zip(((0, 16), (16, 16), (32, 3)), like))
+
+
 def _backward_impl(rs, num_rendered, capacity, extended, means3D, sh, colors_precomp, opacities, scales, rotations,
                    cov3Ds_precomp, shs_language, language_feature_precomp, confidence, radii, geom, binning, img,
-                   g_color, g_depth, g_alpha, g_feature):
+                   g_color, g_depth, g_alpha, g_feature, camera=()):
+    """camera: () or the (shape, dtype) of the viewmatrix, projmatrix and campos tensors whose gradients are wanted;
+    the gradients are appended to the returned tuple."""
     dev = means3D.device
     P = means3D.shape[0]
     keep = []
@@ -261,13 +270,18 @@ def _backward_impl(rs, num_rendered, capacity, extended, means3D, sh, colors_pre
             ("colors", (P, 3), has(colors_precomp)), ("scales", (P, 3), has(scales)), ("rots", (P, 4), has(rotations)),
             ("cov", (P, 6), has(cov3Ds_precomp)), ("feat", (P, 3), extended and has(language_feature_precomp)),
             ("shl", tuple(shs_language.shape) if has(shs_language) else (P, 3), extended and has(shs_language)),
-            ("scratch", (P, 16), P > 0)]
+            ("scratch", (P, 16), P > 0),
+            ("cam", (35,), bool(camera)),
+            ("cam_scratch", (int(lib.b200gs_camera_scratch_bytes(P)) // 4,), bool(camera) and P > 0)]
     shapes = [shp for _, shp, on in want if on]
     views = iter(_carve(torch.empty((max(_carve_size(shapes), 1),), **f32), shapes))
     got = {name: (next(views) if on else None) for name, _, on in want}
     d_means3D, d_means2D, d_opac, d_sh, d_colors = got["means3D"], got["means2D"], got["opac"], got["sh"], got["colors"]
     d_scales, d_rots, d_cov, d_feat, d_shl, scratch = got["scales"], got["rots"], got["cov"], got["feat"], got["shl"], got["scratch"]
     if P == 0:
+        if camera:
+            got["cam"].zero_()
+            return (d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat) + _camera_grads(got["cam"], camera)
         return d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat
 
     g = Gaussians()
@@ -287,16 +301,27 @@ def _backward_impl(rs, num_rendered, capacity, extended, means3D, sh, colors_pre
     gr.dL_dmeans3D, gr.dL_dmeans2D, gr.dL_dshs, gr.dL_dcolors = _ptr(d_means3D), _ptr(d_means2D), _ptr(d_sh), _ptr(d_colors)
     gr.dL_dopacities, gr.dL_dscales, gr.dL_drotations, gr.dL_dcov3D = _ptr(d_opac), _ptr(d_scales), _ptr(d_rots), _ptr(d_cov)
     gr.dL_dfeatures, gr.dL_dshs_language, gr.scratch = _ptr(d_feat), _ptr(d_shl), scratch.data_ptr()
-    check(lib.b200gs_backward(C.byref(v), C.byref(g), radii.data_ptr(), C.byref(ws), C.c_int64(capacity), C.byref(go),
-                              C.byref(gr), _stream(dev)))
+    if not camera:
+        check(lib.b200gs_backward(C.byref(v), C.byref(g), radii.data_ptr(), C.byref(ws), C.c_int64(capacity), C.byref(go),
+                                  C.byref(gr), _stream(dev)))
+        del keep
+        return d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat
+    cam = got["cam"]
+    cg = CameraGrads()
+    cg.dL_dviewmatrix, cg.dL_dprojmatrix, cg.dL_dcampos = cam.data_ptr(), cam[16:].data_ptr(), cam[32:].data_ptr()
+    cg.scratch = got["cam_scratch"].data_ptr()
+    check(lib.b200gs_backward_camera(C.byref(v), C.byref(g), radii.data_ptr(), C.byref(ws), C.c_int64(capacity), C.byref(go),
+                                     C.byref(gr), C.byref(cg), _stream(dev)))
     del keep
-    return d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat
+    return (d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat) + _camera_grads(cam, camera)
 
 
 class _RasterizeGaussians(torch.autograd.Function):
     @staticmethod
     def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
-                shs_language, language_feature_precomp, raster_settings, extended):
+                shs_language, language_feature_precomp, raster_settings, extended, *camera):
+        """camera: () or (viewmatrix, projmatrix, campos) -- the settings' own tensors, passed again so that autograd
+        tracks them; backward then also returns their gradients."""
         rs = raster_settings
         confidence = getattr(rs, "confidence", None)
         args = (rs, means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, shs_language,
@@ -315,6 +340,7 @@ class _RasterizeGaussians(torch.autograd.Function):
         ctx.raster_settings = rs
         ctx.num_rendered, ctx.capacity, ctx.extended = num_rendered, capacity, extended
         ctx.confidence = confidence
+        ctx.camera = tuple((t.shape, t.dtype) for t in camera)
         ctx.save_for_backward(colors_precomp, means3D, scales, rotations, cov3Ds_precomp, radii, sh, opacities,
                               shs_language, language_feature_precomp, geom, binning, img)
         ctx.mark_non_differentiable(radii)
@@ -333,7 +359,7 @@ class _RasterizeGaussians(torch.autograd.Function):
             g_color, g_depth, g_alpha, g_feature = grad_outs[0], None, None, None
         args = (rs, ctx.num_rendered, ctx.capacity, ctx.extended, means3D, sh, colors_precomp, opacities, scales,
                 rotations, cov3Ds_precomp, shs_language, language_feature_precomp, ctx.confidence, radii, geom,
-                binning, img, g_color, g_depth, g_alpha, g_feature)
+                binning, img, g_color, g_depth, g_alpha, g_feature, ctx.camera)
         if rs.debug:
             cpu_args = _cpu_deep_copy_tuple(args[1:])
             try:
@@ -344,17 +370,23 @@ class _RasterizeGaussians(torch.autograd.Function):
                 raise ex
         else:
             grads = _backward_impl(*args)
-        d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat = grads
-        # order of forward()'s inputs (reference order + the two SDP-GS tensors + settings + mode flag)
-        return (d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat, None, None)
+        d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat = grads[:10]
+        # order of forward()'s inputs (reference order + the two SDP-GS tensors + settings + mode flag + camera tensors)
+        return (d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat, None, None) + tuple(grads[10:])
 
 
 def rasterize_gaussians(means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
                         raster_settings, shs_language=None, language_feature_precomp=None, extended=False):
+    """The camera is differentiated when grad mode is on and any of the settings' viewmatrix / projmatrix / campos
+    tensors requires grad (pose refinement); otherwise exactly the vanilla backward runs."""
     empty = lambda t: torch.Tensor([]) if t is None else t
+    rs = raster_settings
+    camera = (rs.viewmatrix, rs.projmatrix, rs.campos)
+    if not (torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.requires_grad for t in camera)):
+        camera = ()
     return _RasterizeGaussians.apply(means3D, means2D, empty(sh), empty(colors_precomp), opacities, empty(scales),
                                      empty(rotations), empty(cov3Ds_precomp), empty(shs_language),
-                                     empty(language_feature_precomp), raster_settings, bool(extended))
+                                     empty(language_feature_precomp), raster_settings, bool(extended), *camera)
 
 
 def mark_visible(positions, viewmatrix, projmatrix):
@@ -416,10 +448,13 @@ class RasterSession:
 
     def __init__(self, raster_settings, *, means3D, opacities, shs=None, colors_precomp=None, scales=None,
                  rotations=None, cov3D_precomp=None, shs_language=None, language_feature_precomp=None,
-                 extended=False, capacity, grads_out=None, with_backward=True, grad_scatter=None, live_count=None):
+                 extended=False, capacity, grads_out=None, with_backward=True, grad_scatter=None, live_count=None,
+                 camera_grads=False):
         """live_count: optional uint32/int32 device tensor of one element -- the number of live rows of capacity-sized
         parameter buffers (b200gs_gaussians_t.live_count); rows past it are culled, so the Gaussian count can change on the
-        device without touching this session or its captured graph."""
+        device without touching this session or its captured graph.
+        camera_grads: backward() also writes the gradients w.r.t. the settings' camera into the static tensors
+        self.camera_grads = {"viewmatrix": [4,4], "projmatrix": [4,4], "campos": [3]} (b200gs_backward_camera)."""
         rs = raster_settings
         self.rs, self.extended, self.capacity = rs, bool(extended), int(capacity)
         dev = means3D.device
@@ -465,6 +500,14 @@ class RasterSession:
         ws.binning, ws.binning_bytes = self.binning.data_ptr(), self.binning.numel()
         self.graph = None
         self.with_backward = with_backward
+        self.camera_grads, self.cg = None, None
+        if camera_grads and with_backward:
+            cam = torch.empty((64 + lib.b200gs_camera_scratch_bytes(P) // 4,), **f32)  # 35 outputs, then the scratch
+            self.camera_grads = dict(viewmatrix=cam[0:16].view(4, 4), projmatrix=cam[16:32].view(4, 4), campos=cam[32:35])
+            cg = self.cg = CameraGrads()
+            cg.dL_dviewmatrix, cg.dL_dprojmatrix, cg.dL_dcampos = cam.data_ptr(), cam[16:].data_ptr(), cam[32:].data_ptr()
+            cg.scratch = cam[64:].data_ptr()
+            self._keep.append(cam)
         if not with_backward:
             ws.persistent = 1
             check(lib.b200gs_workspace_init(C.byref(ws), P, None, _stream(dev)))
@@ -506,6 +549,11 @@ class RasterSession:
                                  C.c_int64(self.capacity), _stream()))
 
     def backward(self):
+        if self.cg is not None:
+            check(lib.b200gs_backward_camera(C.byref(self.v), C.byref(self.g), self.radii.data_ptr(), C.byref(self.ws),
+                                             C.c_int64(self.capacity), C.byref(self.go), C.byref(self.gr), C.byref(self.cg),
+                                             _stream()))
+            return
         check(lib.b200gs_backward(C.byref(self.v), C.byref(self.g), self.radii.data_ptr(), C.byref(self.ws),
                                   C.c_int64(self.capacity), C.byref(self.go), C.byref(self.gr), _stream()))
 

@@ -381,14 +381,37 @@ int b200gs_forward_status(const b200gs_workspace_t* ws, void* stream_, int64_t* 
 	return 0;
 }
 
+size_t b200gs_camera_scratch_bytes(int32_t P) { return camera_scratch_bytes(P); }
+int64_t b200gs_camera_grads_abi_size(void) { return (int64_t)sizeof(b200gs_camera_grads_t); }
+
 int b200gs_backward(const b200gs_view_t* v, const b200gs_gaussians_t* g, const int32_t* radii,
                     const b200gs_workspace_t* ws, int64_t capacity, const b200gs_grad_outputs_t* gout,
-                    const b200gs_grads_t* grads, void* stream_) {
+                    const b200gs_grads_t* grads, void* stream) {
+	return b200gs_backward_camera(v, g, radii, ws, capacity, gout, grads, nullptr, stream);
+}
+
+int b200gs_backward_camera(const b200gs_view_t* v, const b200gs_gaussians_t* g, const int32_t* radii,
+                           const b200gs_workspace_t* ws, int64_t capacity, const b200gs_grad_outputs_t* gout,
+                           const b200gs_grads_t* grads, const b200gs_camera_grads_t* cam, void* stream_) {
 	RasterPlan pl;
 	if (int e = validate(pl, v, g, ws, capacity)) return e;
 	if (!gout || !grads) return fail(B200GS_E_ARG, "null gradient structs");
+	if (cam) {
+		if (!cam->dL_dviewmatrix || !cam->dL_dprojmatrix || !cam->dL_dcampos || !cam->scratch)
+			return fail(B200GS_E_ARG, "camera gradients: dL_dviewmatrix, dL_dprojmatrix, dL_dcampos and scratch are required");
+		if (grads->scatter_bases)
+			return fail(B200GS_E_ARG, "camera gradients are not supported together with the gradient scatter (scatter_bases)");
+	}
 	const int P = g->P;
-	if (P == 0) return 0;  // rasterize_points.cu:161
+	if (P == 0) {  // rasterize_points.cu:161; the camera gradients of an empty scene are zero
+		if (!cam) return 0;
+		cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+		cudaError_t e = cudaMemsetAsync(cam->dL_dviewmatrix, 0, 16 * sizeof(float), stream);
+		if (e == cudaSuccess) e = cudaMemsetAsync(cam->dL_dprojmatrix, 0, 16 * sizeof(float), stream);
+		if (e == cudaSuccess) e = cudaMemsetAsync(cam->dL_dcampos, 0, 3 * sizeof(float), stream);
+		if (e != cudaSuccess) return fail(B200GS_E_CUDA, "[CUDA ERROR] zeroing camera gradients: %s", cudaGetErrorString(e));
+		return 0;
+	}
 	if (!radii || !grads->scratch) return fail(B200GS_E_ARG, "radii and scratch are required");
 	if (grads->scatter_bases) {
 		if (grads->scatter_world < 2 || grads->scatter_rank < 0 || grads->scatter_rank >= grads->scatter_world || grads->scatter_shard_rows <= 0 ||
@@ -403,7 +426,7 @@ int b200gs_backward(const b200gs_view_t* v, const b200gs_gaussians_t* g, const i
 	if (!pl.persistent) { StageScope t(stream, ST_MEMSET); cudaMemsetAsync(grec, 0, b200gs_scratch_bytes(P), stream); }
 	{ StageScope t(stream, ST_BLEND_BWD); launch_blend_backward(pl, *gout, grec, stream); }
 	if (int e = check_stage(v, stream, "blend backward")) return e;
-	{ StageScope t(stream, ST_PREPROCESS_BWD); launch_preprocess_backward(pl, *g, radii, grec, *grads, stream); }
+	{ StageScope t(stream, ST_PREPROCESS_BWD); launch_preprocess_backward(pl, *g, radii, grec, *grads, cam, stream); }
 	return check_stage(v, stream, "preprocess backward");
 }
 

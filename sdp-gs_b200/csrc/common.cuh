@@ -136,8 +136,10 @@ struct RasterPlan {
 
 // ---- stage launchers (each enqueues on `stream`) ----
 void launch_preprocess_forward(const RasterPlan& pl, const b200gs_gaussians_t& g, int32_t* radii, cudaStream_t stream);
+// cam != NULL: also the camera gradients (a second, small kernel reduces the per-CTA partials in cam->scratch)
 void launch_preprocess_backward(const RasterPlan& pl, const b200gs_gaussians_t& g, const int32_t* radii, float* grec,
-                                const b200gs_grads_t& gr, cudaStream_t stream);
+                                const b200gs_grads_t& gr, const b200gs_camera_grads_t* cam, cudaStream_t stream);
+size_t camera_scratch_bytes(int P);
 void launch_mark_visible(int P, const float* means3D, const float* viewmatrix, uint8_t* present, cudaStream_t stream);
 
 void launch_depth_order(const RasterPlan& pl, cudaStream_t stream);  // stable sort of Gaussian ids by depth bits

@@ -376,7 +376,17 @@ __device__ __forceinline__ void store3(float* p, size_t i, float a, float b, flo
 	if (p) { p[3 * i] = a; p[3 * i + 1] = b; p[3 * i + 2] = c; }
 }
 
-__global__ void __launch_bounds__(PRE_THREADS) preprocess_backward_kernel(
+// Camera gradients (CAM = true): the 27 entries of viewmatrix / projmatrix / campos the forward reads, per row
+//   [3c + r]       viewmatrix (r, c), r = 0..2, c = 0..3   (storage 4c + r)
+//   [12 + 3c + k]  projmatrix (r, c), r = 0, 1, 3 for k = 0, 1, 2
+//   [24 + k]       campos k
+// Each CTA assigns its sums to a column-major [CAM_TERMS][gridDim.x] scratch, which camera_grad_reduce_kernel reduces.
+// Shared memory allows 5 CTAs per SM; left alone, ptxas gives CAM = true 122 registers (4 CTAs), so it is held to 5
+// (96 registers, 100 bytes of spill stores).  CAM = false keeps no minimum (0): its code is the same as without CAM.
+constexpr int CAM_TERMS = 27;
+
+template <bool CAM>
+__global__ void __launch_bounds__(PRE_THREADS, CAM ? 5 : 0) preprocess_backward_kernel(
 	int P, int D, int M, const float* __restrict__ means3D, const int32_t* __restrict__ radii,
 	const float* __restrict__ shs, const uint8_t* __restrict__ clamped, const float* __restrict__ scales,
 	const float* __restrict__ rotations, float scale_modifier, const float* __restrict__ cov3D_precomp,
@@ -388,7 +398,7 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_backward_kernel(
 	float* __restrict__ dL_dcolors, float* __restrict__ dL_dopac, float* __restrict__ dL_dscales,
 	float* __restrict__ dL_drots, float* __restrict__ dL_dcov3D, float* __restrict__ dL_dfeat,
 	float* __restrict__ dL_dshs_lang, int tma_ok, void* const* __restrict__ scatter_bases, long long scatter_Ps, int scatter_rank,
-	int accumulate, int scatter_tma)
+	int accumulate, int scatter_tma, float* __restrict__ cam_part)
 {
 	// inputs staged as in the forward; the same buffers are reused for the outgoing gradients (a thread only ever
 	// touches its own row), which leave as contiguous bulk stores instead of 12/24/192-byte strided scalar stores
@@ -440,6 +450,11 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_backward_kernel(
 #pragma unroll
 	for (int k = 0; k < 16; k++) shw[k] = 0.f;
 	float dRGB[3] = {0.f, 0.f, 0.f};
+	float cg[CAM_TERMS];  // this row's camera terms (zero unless rendered)
+	if constexpr (CAM) {
+#pragma unroll
+		for (int i = 0; i < CAM_TERMS; i++) cg[i] = 0.f;
+	}
 	if (idx < P && __ldcg(radii + idx) > 0) {
 	ViewConsts vc;
 	load_view(vc, viewmatrix, projmatrix, campos);
@@ -553,7 +568,12 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_backward_kernel(
 		const unsigned cl = __ldcg(clamped + idx);
 		dRGB[0] *= (cl & 1u) ? 0.f : 1.f; dRGB[1] *= (cl & 2u) ? 0.f : 1.f; dRGB[2] *= (cl & 4u) ? 0.f : 1.f;
 		const float dox = mx - vc.campos[0], doy = my - vc.campos[1], doz = mz - vc.campos[2];
-		const float ilen = 1.0f / sqrtf(dox * dox + doy * doy + doz * doz);
+		// The squares below have several uses; the default build rounds each once and fuses none of them into an add.  The
+		// CAM build would fuse some (its extra code changes the compiler's choices), so there they are pinned to that
+		// rounding: the parameter gradients of both builds stay bit-identical.
+		auto sq = [](float a) { if constexpr (CAM) return __fmul_rn(a, a); else return a * a; };
+		auto add = [](float a, float b) { if constexpr (CAM) return __fadd_rn(a, b); else return a + b; };
+		const float ilen = 1.0f / sqrtf(add(add(sq(dox), sq(doy)), sq(doz)));
 		const float x = dox * ilen, y = doy * ilen, z = doz * ilen;
 		const float* sh = sh_staged ? s_sh + li * M * 3 : shs + (size_t)idx * M * 3;
 		float ddir[3] = {0.f, 0.f, 0.f};  // dL/ddir
@@ -582,7 +602,7 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_backward_kernel(
 			const float s1 = shdot(1), s2 = shdot(2), s3d = shdot(3);
 			ddir[0] = -kSH_C1 * s3d; ddir[1] = -kSH_C1 * s1; ddir[2] = kSH_C1 * s2;
 			if (D > 1) {
-				const float xx = x * x, yy = y * y, zz = z * z, xy = x * y, yz = y * z, xz = x * z;
+				const float xx = sq(x), yy = sq(y), zz = sq(z), xy = x * y, yz = y * z, xz = x * z;
 				wr(4, kSH_C2[0] * xy); wr(5, kSH_C2[1] * yz); wr(6, kSH_C2[2] * (2.f * zz - xx - yy));
 				wr(7, kSH_C2[3] * xz); wr(8, kSH_C2[4] * (xx - yy));
 				written = 9;
@@ -611,11 +631,20 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_backward_kernel(
 		}
 		(void)written;
 		// dnormvdv (auxiliary.h:107-117)
-		const float sum2 = dox * dox + doy * doy + doz * doz;
+		const float sum2 = add(add(sq(dox), sq(doy)), sq(doz));
 		const float invsum32 = 1.0f / sqrtf(sum2 * sum2 * sum2);
-		dmean[0] += ((+sum2 - dox * dox) * ddir[0] - doy * dox * ddir[1] - doz * dox * ddir[2]) * invsum32;
-		dmean[1] += (-dox * doy * ddir[0] + (sum2 - doy * doy) * ddir[1] - doz * doy * ddir[2]) * invsum32;
-		dmean[2] += (-dox * doz * ddir[0] - doy * doz * ddir[1] + (sum2 - doz * doz) * ddir[2]) * invsum32;
+		const float nx = (+sum2 - sq(dox)) * ddir[0] - doy * dox * ddir[1] - doz * dox * ddir[2];
+		const float ny = -dox * doy * ddir[0] + (sum2 - sq(doy)) * ddir[1] - doz * doy * ddir[2];
+		const float nz = -dox * doz * ddir[0] - doy * doz * ddir[1] + (sum2 - sq(doz)) * ddir[2];
+		if constexpr (CAM) {
+			// dir = mean - campos.  Here the product n * invsum32 has a second use, so the compiler would round it before
+			// the add; the FMA it contracts to in the default build is pinned, keeping dL/dmean bit-identical to it
+			dmean[0] = __fmaf_rn(nx, invsum32, dmean[0]); dmean[1] = __fmaf_rn(ny, invsum32, dmean[1]);
+			dmean[2] = __fmaf_rn(nz, invsum32, dmean[2]);
+			cg[24] = -(nx * invsum32); cg[25] = -(ny * invsum32); cg[26] = -(nz * invsum32);
+		} else {
+			dmean[0] += nx * invsum32; dmean[1] += ny * invsum32; dmean[2] += nz * invsum32;
+		}
 	}
 
 	o_mean[0] = dmean[0]; o_mean[1] = dmean[1]; o_mean[2] = dmean[2];
@@ -656,6 +685,25 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_backward_kernel(
 		dq.z = 2 * x * (dMt[1][0] + dMt[0][1]) + 2 * r * (dMt[2][0] - dMt[0][2]) + 2 * z * (dMt[1][2] + dMt[2][1]) - 4 * y * (dMt[2][2] + dMt[0][0]);
 		dq.w = 2 * r * (dMt[0][1] - dMt[1][0]) + 2 * x * (dMt[2][0] + dMt[0][2]) + 2 * y * (dMt[1][2] + dMt[2][1]) - 4 * z * (dMt[1][1] + dMt[0][0]);
 		o_rot = dq;
+	}
+	if constexpr (CAM) {
+		// t = A mh (mh = (mean, 1)): dA(r, c) += dt_r mh_c, the depth head's cotangent joining dt_z
+		const float mh[4] = {mx, my, mz, 1.f};
+		const float dt[3] = {dtx, dty, extended ? dtz + dz : dtz};
+		// h = Pm mh, projected as h_r / (h_3 + 1e-7): dPm(r, c) += dh_r mh_c for r = 0, 1, 3
+		const float dh[3] = {dm2x * m_w, dm2y * m_w, -(dm2x * mul1 + dm2y * mul2)};
+#pragma unroll
+		for (int c = 0; c < 4; c++)
+#pragma unroll
+			for (int r = 0; r < 3; r++) { cg[3 * c + r] = dt[r] * mh[c]; cg[12 + 3 * c + r] = dh[r] * mh[c]; }
+		// T = J W with W = A[0:3, 0:3]: T0j = J00 W0j + J02 W2j, T1j = J11 W1j + J12 W2j
+		const float dT0[3] = {dT00, dT01, dT02}, dT1[3] = {dT10, dT11, dT12};
+#pragma unroll
+		for (int j = 0; j < 3; j++) {
+			cg[3 * j] += dT0[j] * J00;
+			cg[3 * j + 1] += dT1[j] * J11;
+			cg[3 * j + 2] += dT0[j] * J02 + dT1[j] * J12;
+		}
 	}
 	}  // rendered Gaussian
 
@@ -739,8 +787,31 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_backward_kernel(
 			else if (dL_drots) { float* r = dL_drots + 4 * (size_t)idx; r[0] = o_rot.x; r[1] = o_rot.y; r[2] = o_rot.z; r[3] = o_rot.w; }
 		}
 	}
+	if constexpr (CAM) {
+		float* s_cam = reinterpret_cast<float*>(s_grec);  // [warp][32] warp sums (every row of s_grec was read before the last barrier)
+		// transposing butterfly: at each step a lane keeps half of its values and adds its partner's copy of that half,
+		// so 32 values (27 terms, zero-padded) need 16 + 8 + 4 + 2 + 1 shuffles and lane l ends with the warp's sum of value l
+		float v[32];
+#pragma unroll
+		for (int i = 0; i < 32; i++) v[i] = i < CAM_TERMS ? cg[i] : 0.f;
+#pragma unroll
+		for (int s = 16; s >= 1; s >>= 1) {
+			const bool hi = (li & s) != 0;
+#pragma unroll
+			for (int i = 0; i < s; i++) {
+				const float send = hi ? v[i] : v[i + s], keep = hi ? v[i + s] : v[i];
+				v[i] = keep + __shfl_xor_sync(0xFFFFFFFFu, send, s);
+			}
+		}
+		s_cam[li] = v[0];
+	}
 	tma_store_fence();
 	__syncthreads();
+	if constexpr (CAM) {  // the CTA's sums, warps added in a fixed order: assigned, so the scratch needs no zeroing
+		const float* s_cam = reinterpret_cast<const float*>(s_grec);
+		if (li < CAM_TERMS)
+			cam_part[(size_t)li * gridDim.x + blockIdx.x] = (s_cam[li] + s_cam[32 + li]) + (s_cam[64 + li] + s_cam[96 + li]);
+	}
 	auto put = [&](float* dst, const float* src, int floats_per_item) {
 		if (dst == nullptr) return;
 		float* g = dst + base * floats_per_item;
@@ -797,7 +868,61 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_backward_kernel(
 	if (full && li == 0) { tma_store_commit(); tma_store_wait_read(); }
 }
 
+// One CTA per output float of b200gs_camera_grads_t (16 viewmatrix, 16 projmatrix, 3 campos, in storage order): the CTA
+// partials of its term summed in float64 in a fixed order; entries the forward never reads are written as zeros.  Each
+// thread keeps CAM_REDUCE_UNROLL loads in flight (46 875 partials per term at 6 M Gaussians: one dependent load per step
+// would make this latency-bound kernel cost more than the per-row arithmetic).
+constexpr int CAM_REDUCE_THREADS = 1024, CAM_REDUCE_UNROLL = 8;
+__global__ void __launch_bounds__(CAM_REDUCE_THREADS) camera_grad_reduce_kernel(
+	const float* cam_part, int nblk, float* __restrict__ dL_dview, float* __restrict__ dL_dproj, float* __restrict__ dL_dcampos)
+{
+	__shared__ double s_sum[CAM_REDUCE_THREADS];
+	pdl_trigger();
+	const int e = blockIdx.x, tid = threadIdx.x;
+	int term = -1;
+	if (e < 16) {
+		const int r = e & 3, c = e >> 2;
+		if (r != 3) term = 3 * c + r;
+	} else if (e < 32) {
+		const int r = (e - 16) & 3, c = (e - 16) >> 2;
+		if (r != 2) term = 12 + 3 * c + (r == 3 ? 2 : r);
+	} else {
+		term = 24 + (e - 32);
+	}
+	pdl_wait();  // the partials are written by the preprocess backward just before
+	double acc = 0.0;
+	if (term >= 0) {
+		const float* p = cam_part + (size_t)term * nblk;
+		for (int i0 = tid; i0 < nblk; i0 += CAM_REDUCE_THREADS * CAM_REDUCE_UNROLL) {
+			float x[CAM_REDUCE_UNROLL];
+#pragma unroll
+			for (int u = 0; u < CAM_REDUCE_UNROLL; u++) {
+				const int i = i0 + u * CAM_REDUCE_THREADS;
+				x[u] = i < nblk ? __ldcg(p + i) : 0.f;
+			}
+#pragma unroll
+			for (int u = 0; u < CAM_REDUCE_UNROLL; u++) acc += (double)x[u];
+		}
+	}
+	s_sum[tid] = acc;
+	__syncthreads();
+#pragma unroll
+	for (int w = CAM_REDUCE_THREADS / 2; w > 0; w >>= 1) {
+		if (tid < w) s_sum[tid] += s_sum[tid + w];
+		__syncthreads();
+	}
+	if (tid == 0) {
+		float* out = e < 16 ? dL_dview + e : e < 32 ? dL_dproj + (e - 16) : dL_dcampos + (e - 32);
+		*out = (float)s_sum[0];
+	}
+}
+
 }  // namespace
+
+size_t camera_scratch_bytes(int P) {
+	const size_t nblk = P > 0 ? ((size_t)P + PRE_THREADS - 1) / PRE_THREADS : 1;
+	return nblk * CAM_TERMS * sizeof(float);
+}
 
 void launch_preprocess_forward(const RasterPlan& pl, const b200gs_gaussians_t& g, int32_t* radii, cudaStream_t stream) {
 	const b200gs_view_t& v = *pl.v;
@@ -818,9 +943,10 @@ void launch_preprocess_forward(const RasterPlan& pl, const b200gs_gaussians_t& g
 }
 
 void launch_preprocess_backward(const RasterPlan& pl, const b200gs_gaussians_t& g, const int32_t* radii, float* grec,
-                                const b200gs_grads_t& gr, cudaStream_t stream) {
+                                const b200gs_grads_t& gr, const b200gs_camera_grads_t* cam, cudaStream_t stream) {
 	const b200gs_view_t& v = *pl.v;
 	const int P = g.P;
+	const unsigned nblk = (P + PRE_THREADS - 1) / PRE_THREADS;
 	const float focal_y = v.height / (2.0f * v.tan_fovy);
 	const float focal_x = v.width / (2.0f * v.tan_fovx);
 	const auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
@@ -829,13 +955,17 @@ void launch_preprocess_backward(const RasterPlan& pl, const b200gs_gaussians_t& 
 	                   al16(gr.dL_dshs) && al16(gr.dL_dcolors) && al16(gr.dL_dscales) && al16(gr.dL_dcov3D) && al16(gr.dL_dfeatures) &&
 	                   al16(gr.dL_dshs_language);
 	const int scatter_tma = knob_int(KNOB_SCATTER_TMA, 1);  // 0: plain stores to the peer staging blocks (A/B)
-	launch(PDL_PRE_BWD, preprocess_backward_kernel, dim3((P + PRE_THREADS - 1) / PRE_THREADS), dim3(PRE_THREADS), 0, stream,
+	float* cam_part = cam ? reinterpret_cast<float*>(cam->scratch) : nullptr;
+	launch(PDL_PRE_BWD, cam ? preprocess_backward_kernel<true> : preprocess_backward_kernel<false>, dim3(nblk), dim3(PRE_THREADS), 0, stream,
 		P, v.sh_degree, v.sh_coeffs, g.means3D, radii, g.shs, pl.gs.clamped, g.scales, g.rotations, v.scale_modifier,
 		g.cov3D_precomp, g.language_feature_precomp, g.shs_language, g.confidence, v.viewmatrix, v.projmatrix,
 		v.campos, focal_x, focal_y, v.tan_fovx, v.tan_fovy, v.extended, reinterpret_cast<float4*>(grec), pl.persistent ? 1 : 0,
 		gr.dL_dmeans3D, gr.dL_dmeans2D, gr.dL_dshs, gr.dL_dcolors, gr.dL_dopacities, gr.dL_dscales,
 		gr.dL_drotations, gr.dL_dcov3D, gr.dL_dfeatures, gr.dL_dshs_language, tma_ok, gr.scatter_bases,
-		(long long)gr.scatter_shard_rows, (int)gr.scatter_rank, (int)gr.accumulate, scatter_tma);
+		(long long)gr.scatter_shard_rows, (int)gr.scatter_rank, (int)gr.accumulate, scatter_tma, cam_part);
+	if (cam)
+		launch(PDL_PRE_BWD, camera_grad_reduce_kernel, dim3(35), dim3(CAM_REDUCE_THREADS), 0, stream, (const float*)cam_part, (int)nblk,
+		       cam->dL_dviewmatrix, cam->dL_dprojmatrix, cam->dL_dcampos);
 }
 
 void launch_mark_visible(int P, const float* means3D, const float* viewmatrix, uint8_t* present, cudaStream_t stream) {

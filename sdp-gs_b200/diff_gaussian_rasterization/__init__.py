@@ -13,6 +13,9 @@ Both API shapes of SURVEY.md §8(b) are served by the same classes:
 
 The SDP-GS shape is selected when the settings carry `include_feature`/`confidence` or when either
 feature argument is passed.
+
+Beyond the reference, the camera is differentiable: when the settings' `viewmatrix`, `projmatrix` or
+`campos` requires grad, backward also returns their gradients (pose refinement, INTEGRATION.md).
 """
 from typing import NamedTuple, Optional
 

@@ -20,7 +20,9 @@ from diff_gaussian_rasterization import GaussianRasterizationSettings, GaussianR
 
 def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, opt, scaling_modifier=1.0, override_color=None,
            override_language=None):
-    """Render the scene.  Background tensor (bg_color) must be on the GPU."""
+    """Render the scene.  Background tensor (bg_color) must be on the GPU.  When the camera's
+    world_view_transform / full_proj_transform / camera_center require grad (a learnable pose), the
+    backward also differentiates them."""
     xyz = pc.get_xyz
     # zero tensor whose gradient receives the 2D (screen-space) mean gradients (gaussian_renderer/__init__.py:217-221)
     screenspace_points = torch.zeros_like(xyz, dtype=xyz.dtype, requires_grad=True, device=xyz.device) + 0
