@@ -9,6 +9,7 @@ PyTorch is only used for device memory, streams and autograd plumbing.
 from __future__ import annotations
 
 import ctypes as C
+import math
 
 import torch
 
@@ -80,26 +81,16 @@ def _f32c(t, name):
     return t if t.is_contiguous() else t.contiguous()
 
 
-def _carve(flat, shapes, align=64):
-    """Views of one flat allocation (one allocator call instead of one per output); `align` in elements."""
-    out, off = [], 0
+def _carve(shapes, align=64, **opts):
+    """Views of one new flat allocation (one allocator call instead of one per tensor), each starting at a multiple of
+    `align` elements."""
+    spans, tot = [], 0
     for shp in shapes:
-        n = 1
-        for d in shp:
-            n *= d
-        out.append(flat[off:off + n].view(shp))
-        off += (n + align - 1) // align * align
-    return out
-
-
-def _carve_size(shapes, align=64):
-    tot = 0
-    for shp in shapes:
-        n = 1
-        for d in shp:
-            n *= d
+        n = math.prod(shp)
+        spans.append((tot, n))
         tot += (n + align - 1) // align * align
-    return tot
+    flat = torch.empty((max(tot, 1),), **opts)
+    return [flat[o:o + n].view(shp) for (o, n), shp in zip(spans, shapes)]
 
 
 def _stream(device=None):
@@ -108,8 +99,18 @@ def _stream(device=None):
     return C.c_void_p(torch._C._cuda_getCurrentRawStream(idx))
 
 
-def _cpu_deep_copy_tuple(args):
-    return tuple(a.detach().cpu().clone() if isinstance(a, torch.Tensor) else a for a in args)
+def _with_snapshot(rs, dump, message, fn, *args):
+    """fn(rs, *args); in debug mode, as in the reference, a CPU copy of `args` taken before the call is saved to `dump` if
+    it raises."""
+    if not rs.debug:
+        return fn(rs, *args)
+    cpu_args = tuple(a.detach().cpu().clone() if isinstance(a, torch.Tensor) else a for a in args)  # before they can be corrupted
+    try:
+        return fn(rs, *args)
+    except Exception:
+        torch.save(cpu_args, dump)
+        print(message)
+        raise
 
 
 _WS_BYTES = {}
@@ -122,11 +123,6 @@ def _ws_bytes(P, W, H):
     if v is None:
         v = _WS_BYTES[k] = (int(lib.b200gs_geom_bytes(P)), int(lib.b200gs_image_bytes(W, H)))
     return v
-
-
-class _State:
-    """What forward leaves behind for backward / inspection."""
-    __slots__ = ("view", "gauss", "keep", "P", "W", "H", "capacity", "num_rendered", "extended")
 
 
 def _build_view(rs, P, M, extended, keep):
@@ -167,29 +163,118 @@ def _cached_view(rs, P, M, extended, keep):
     return v
 
 
-def _forward_impl(rs, means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, shs_language,
-                  language_feature_precomp, confidence, extended):
+_GRADS = ("means3D", "means2D", "shs", "colors_precomp", "opacities", "scales", "rotations", "cov3D", "shs_language",
+          "features")  # the gradients, in the order of the autograd op's inputs
+
+
+def _gaussians(means3D, shs, colors_precomp, opacities, scales, rotations, cov3D_precomp, shs_language,
+               language_feature_precomp, confidence, live_count=None):
+    """The per-Gaussian inputs as the kernels read them -- float32, contiguous CUDA tensors (the same tensor where it
+    already is one), None where absent or empty, keyed like the arguments -- and the Gaussians struct over them."""
     if means3D.dim() != 2 or means3D.shape[1] != 3:
         raise RuntimeError("means3D must have dimensions (num_points, 3)")  # rasterize_points.cu:57-59
-    dev = means3D.device
-    P = means3D.shape[0]
-    H, W = int(rs.image_height), int(rs.image_width)
-    keep = []
-    means3D = _f32c(means3D, "means3D")
-    sh, colors_precomp = _f32c(sh, "shs"), _f32c(colors_precomp, "colors_precomp")
-    opacities = _f32c(opacities, "opacities")
-    scales, rotations = _f32c(scales, "scales"), _f32c(rotations, "rotations")
-    cov3Ds_precomp = _f32c(cov3Ds_precomp, "cov3D_precomp")
-    shs_language = _f32c(shs_language, "shs_language")
-    language_feature_precomp = _f32c(language_feature_precomp, "language_feature_precomp")
-    confidence = _f32c(confidence, "confidence")
-    M = 0 if sh is None else int(sh.shape[1])  # rasterize_points.cu:83-87
+    inputs = dict(means3D=_f32c(means3D, "means3D"), shs=_f32c(shs, "shs"), colors_precomp=_f32c(colors_precomp, "colors_precomp"),
+                  opacities=_f32c(opacities, "opacities"), scales=_f32c(scales, "scales"), rotations=_f32c(rotations, "rotations"),
+                  cov3D_precomp=_f32c(cov3D_precomp, "cov3D_precomp"), shs_language=_f32c(shs_language, "shs_language"),
+                  language_feature_precomp=_f32c(language_feature_precomp, "language_feature_precomp"),
+                  confidence=_f32c(confidence, "confidence"))
+    if live_count is not None and (live_count.device != means3D.device or live_count.numel() != 1
+                                   or live_count.dtype not in (torch.int32, torch.uint32)):
+        raise RuntimeError("live_count must be a one-element int32/uint32 tensor on the session's device")
+    return inputs, _gaussians_struct(means3D.shape[0], inputs, live_count)
 
+
+def _gaussians_struct(P, inputs, live_count=None):
+    """The Gaussians struct over tensors _gaussians returned (the backward's saved ones)."""
     g = Gaussians()
     g.P = P
-    g.means3D, g.shs, g.colors_precomp, g.opacities = _ptr(means3D), _ptr(sh), _ptr(colors_precomp), _ptr(opacities)
-    g.scales, g.rotations, g.cov3D_precomp = _ptr(scales), _ptr(rotations), _ptr(cov3Ds_precomp)
-    g.language_feature_precomp, g.shs_language, g.confidence = _ptr(language_feature_precomp), _ptr(shs_language), _ptr(confidence)
+    for k, t in inputs.items():
+        setattr(g, k, None if t is None else t.data_ptr())
+    if live_count is not None:
+        g.live_count = live_count.data_ptr()
+    return g
+
+
+def _workspace(geom, img, binning=None):
+    ws = Workspace()
+    ws.geom, ws.geom_bytes, ws.image, ws.image_bytes = geom.data_ptr(), geom.numel(), img.data_ptr(), img.numel()
+    if binning is not None:
+        ws.binning, ws.binning_bytes = binning.data_ptr(), binning.numel()
+    return ws
+
+
+def _grad_buffers(inputs, P, device, extended, camera=False, given=None):
+    """What a backward over `inputs` (as _gaussians returns them) writes, as views of one float32 allocation: the
+    gradients under the keys of _GRADS (None where the input is absent), the per-Gaussian "scratch" and, with `camera`, the
+    35 floats of CameraGrads ("camera") followed by their "camera_scratch".  The kernels write every element (zeros where
+    radii == 0): nothing is filled.  `given` maps gradient keys to caller-owned buffers used instead of carved ones."""
+    i, given = inputs, given or {}
+    has = lambda k: i[k] is not None
+    M = int(i["shs"].shape[1]) if has("shs") else 0
+    want = [("means3D", (P, 3), True), ("means2D", (P, 3), True), ("shs", (P, M, 3), has("shs")),
+            ("colors_precomp", (P, 3), has("colors_precomp")), ("opacities", (P, 1), True),
+            ("scales", (P, 3), has("scales")), ("rotations", (P, 4), has("rotations")),
+            ("cov3D", (P, 6), has("cov3D_precomp")),
+            ("shs_language", tuple(i["shs_language"].shape) if has("shs_language") else None, extended and has("shs_language")),
+            ("features", (P, 3), extended and has("language_feature_precomp")),
+            ("scratch", (max(P, 1), 16), True)]  # b200gs_scratch_bytes(P)
+    if camera:
+        want += [("camera", (35,), True), ("camera_scratch", (int(lib.b200gs_camera_scratch_bytes(P)) // 4,), True)]
+    out, carve = dict.fromkeys(_GRADS), []
+    for k, shape, on in want:
+        if not on:
+            continue
+        t = given.get(k)
+        if t is None:
+            carve.append((k, shape))
+        elif not t.is_contiguous() or t.dtype != torch.float32:
+            raise RuntimeError(f"grads_out[{k}] must be a contiguous float32 tensor")
+        else:
+            out[k] = t
+    out.update(zip([k for k, _ in carve], _carve([shape for _, shape in carve], dtype=torch.float32, device=device)))
+    return out
+
+
+def _grads_struct(grads):
+    gr = Grads()
+    gr.dL_dmeans3D, gr.dL_dmeans2D, gr.dL_dshs, gr.dL_dcolors = _ptr(grads["means3D"]), _ptr(grads["means2D"]), _ptr(grads["shs"]), _ptr(grads["colors_precomp"])
+    gr.dL_dopacities, gr.dL_dscales, gr.dL_drotations, gr.dL_dcov3D = _ptr(grads["opacities"]), _ptr(grads["scales"]), _ptr(grads["rotations"]), _ptr(grads["cov3D"])
+    gr.dL_dfeatures, gr.dL_dshs_language, gr.scratch = _ptr(grads["features"]), _ptr(grads["shs_language"]), grads["scratch"].data_ptr()
+    return gr
+
+
+def _camera_struct(out, scratch):
+    """CameraGrads over `out`, the 35 floats (viewmatrix, projmatrix, campos, each in storage order), and its scratch."""
+    cg = CameraGrads()
+    cg.dL_dviewmatrix, cg.dL_dprojmatrix, cg.dL_dcampos = out.data_ptr(), out[16:].data_ptr(), out[32:].data_ptr()
+    cg.scratch = scratch.data_ptr()
+    return cg
+
+
+def _backward(v, g, radii, ws, capacity, go, gr, cg, stream):
+    """b200gs_backward, or b200gs_backward_camera when camera gradients are wanted (cg is not None)."""
+    args = (C.byref(v), C.byref(g), radii.data_ptr(), C.byref(ws), C.c_int64(capacity), C.byref(go), C.byref(gr))
+    if cg is None:
+        check(lib.b200gs_backward(*args, stream))
+    else:
+        check(lib.b200gs_backward_camera(*args, C.byref(cg), stream))
+
+
+def _forward_impl(rs, means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, shs_language,
+                  language_feature_precomp, confidence, extended):
+    return _forward(rs, means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, shs_language,
+                    language_feature_precomp, confidence, extended)[1]
+
+
+def _forward(rs, means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, shs_language,
+             language_feature_precomp, confidence, extended):
+    """(the per-Gaussian tensors the kernels read, as _gaussians returns them; the result of _forward_impl)"""
+    inputs, g = _gaussians(means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, shs_language,
+                           language_feature_precomp, confidence)
+    dev, P = means3D.device, g.P
+    H, W = int(rs.image_height), int(rs.image_width)
+    keep = []
+    M = 0 if inputs["shs"] is None else int(inputs["shs"].shape[1])  # rasterize_points.cu:83-87
     v = _cached_view(rs, P, M, extended, keep)
 
     f32 = dict(dtype=torch.float32, device=dev)
@@ -207,44 +292,43 @@ def _forward_impl(rs, means3D, sh, colors_precomp, opacities, scales, rotations,
     gb, ib = _ws_bytes(P, W, H)
     wsbuf = torch.empty((gb + ib,), dtype=torch.uint8, device=dev)  # geom | image in one allocation (both 256-byte multiples)
     geom, img = wsbuf[:gb], wsbuf[gb:]
-    ws = Workspace()
-    ws.geom, ws.geom_bytes, ws.image, ws.image_bytes = geom.data_ptr(), gb, img.data_ptr(), ib
-    stream = _stream(dev)
     if P == 0:  # rasterize_points.cu:81: nothing is launched for an empty scene, outputs are zeros
         color.zero_()
         if extended:
             depth.zero_(); alpha.zero_(); feature.zero_()
         binning = torch.empty((0,), dtype=torch.uint8, device=dev)
-        return 0, 0, color, depth, alpha, feature, radii, geom, binning, img
+        return inputs, (0, 0, color, depth, alpha, feature, radii, geom, binning, img)
+    ws = _workspace(geom, img)
+    stream = _stream(dev)
     auto_key = None
     if _CAPACITY == "auto":
         _check_pending()
         auto_key = (P, W, H, str(dev))
-    if _CAPACITY is None or (auto_key is not None and auto_key not in _AUTO):
+    exact = _CAPACITY is None or (auto_key is not None and auto_key not in _AUTO)
+    if exact:  # preprocess, read num_rendered back, size the binning workspace exactly
         n = C.c_int64(0)
         check(lib.b200gs_forward_preprocess(C.byref(v), C.byref(g), C.byref(o), C.byref(ws), stream, C.byref(n)))
         num_rendered, capacity = int(n.value), int(n.value)
         if auto_key is not None:
             _AUTO[auto_key] = int(n.value * 1.3) + 4096
             auto_key = None  # exact this time, nothing to verify
-        binning = torch.empty((lib.b200gs_binning_bytes(capacity, W, H),), dtype=torch.uint8, device=dev)
-        ws.binning, ws.binning_bytes = binning.data_ptr(), binning.numel()
-        check(lib.b200gs_forward_render(C.byref(v), C.byref(g), C.byref(o), C.byref(ws), C.c_int64(capacity), stream))
+        bb = int(lib.b200gs_binning_bytes(capacity, W, H))
     else:  # capacity known up front: one call, no host synchronization
         num_rendered, capacity = -1, int(_AUTO[auto_key] if auto_key is not None else _CAPACITY)
         bb = _BIN_BYTES.get((capacity, W, H))
         if bb is None:
             bb = _BIN_BYTES[(capacity, W, H)] = int(lib.b200gs_binning_bytes(capacity, W, H))
-        binning = torch.empty((bb,), dtype=torch.uint8, device=dev)
-        ws.binning, ws.binning_bytes = binning.data_ptr(), bb
-        check(lib.b200gs_forward(C.byref(v), C.byref(g), C.byref(o), C.byref(ws), C.c_int64(capacity), stream))
+    binning = torch.empty((bb,), dtype=torch.uint8, device=dev)
+    ws.binning, ws.binning_bytes = binning.data_ptr(), bb
+    render = lib.b200gs_forward_render if exact else lib.b200gs_forward
+    check(render(C.byref(v), C.byref(g), C.byref(o), C.byref(ws), C.c_int64(capacity), stream))
     if auto_key is not None:  # asynchronous read-back of {num_rendered, overflow}; looked at by a later call
         ev, host = _FREE_STATUS.pop() if _FREE_STATUS else (torch.cuda.Event(), torch.empty((16,), dtype=torch.uint8, pin_memory=True))
         host.copy_(geom[:16], non_blocking=True)
         ev.record()
         _PENDING.append((ev, host, auto_key))
     del keep
-    return num_rendered, capacity, color, depth, alpha, feature, radii, geom, binning, img
+    return inputs, (num_rendered, capacity, color, depth, alpha, feature, radii, geom, binning, img)
 
 
 def _camera_grads(flat, like):
@@ -257,63 +341,29 @@ def _camera_grads(flat, like):
 def _backward_impl(rs, num_rendered, capacity, extended, means3D, sh, colors_precomp, opacities, scales, rotations,
                    cov3Ds_precomp, shs_language, language_feature_precomp, confidence, radii, geom, binning, img,
                    g_color, g_depth, g_alpha, g_feature, camera=()):
-    """camera: () or the (shape, dtype) of the viewmatrix, projmatrix and campos tensors whose gradients are wanted;
-    the gradients are appended to the returned tuple."""
-    dev = means3D.device
-    P = means3D.shape[0]
-    keep = []
-    M = 0 if (sh is None or sh.numel() == 0) else int(sh.shape[1])
-    f32 = dict(dtype=torch.float32, device=dev)
-    has = lambda t: t is not None and t.numel() != 0
-    # every buffer is fully written by the kernels (zeros where radii == 0): no torch.zeros fills.  One allocation, carved.
-    want = [("means3D", (P, 3), True), ("means2D", (P, 3), True), ("opac", (P, 1), True), ("sh", (P, M, 3), has(sh)),
-            ("colors", (P, 3), has(colors_precomp)), ("scales", (P, 3), has(scales)), ("rots", (P, 4), has(rotations)),
-            ("cov", (P, 6), has(cov3Ds_precomp)), ("feat", (P, 3), extended and has(language_feature_precomp)),
-            ("shl", tuple(shs_language.shape) if has(shs_language) else (P, 3), extended and has(shs_language)),
-            ("scratch", (P, 16), P > 0),
-            ("cam", (35,), bool(camera)),
-            ("cam_scratch", (int(lib.b200gs_camera_scratch_bytes(P)) // 4,), bool(camera) and P > 0)]
-    shapes = [shp for _, shp, on in want if on]
-    views = iter(_carve(torch.empty((max(_carve_size(shapes), 1),), **f32), shapes))
-    got = {name: (next(views) if on else None) for name, _, on in want}
-    d_means3D, d_means2D, d_opac, d_sh, d_colors = got["means3D"], got["means2D"], got["opac"], got["sh"], got["colors"]
-    d_scales, d_rots, d_cov, d_feat, d_shl, scratch = got["scales"], got["rots"], got["cov"], got["feat"], got["shl"], got["scratch"]
-    if P == 0:
-        if camera:
-            got["cam"].zero_()
-            return (d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat) + _camera_grads(got["cam"], camera)
-        return d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat
-
-    g = Gaussians()
-    g.P = P
-    g.means3D, g.shs, g.colors_precomp, g.opacities = _ptr(means3D), _ptr(sh), _ptr(colors_precomp), _ptr(opacities)
-    g.scales, g.rotations, g.cov3D_precomp = _ptr(scales), _ptr(rotations), _ptr(cov3Ds_precomp)
-    g.language_feature_precomp, g.shs_language, g.confidence = _ptr(language_feature_precomp), _ptr(shs_language), _ptr(confidence)
-    v = _cached_view(rs, P, M, extended, keep)
-    ws = Workspace()
-    ws.geom, ws.geom_bytes, ws.image, ws.image_bytes = geom.data_ptr(), geom.numel(), img.data_ptr(), img.numel()
-    ws.binning, ws.binning_bytes = binning.data_ptr(), binning.numel()
-    go = GradOutputs()
-    gc = _f32c(g_color, "grad color")
-    gd, ga, gf = _f32c(g_depth, "grad depth"), _f32c(g_alpha, "grad alpha"), _f32c(g_feature, "grad feature")
-    go.dL_dcolor, go.dL_ddepth, go.dL_dalpha, go.dL_dfeature = _ptr(gc), _ptr(gd), _ptr(ga), _ptr(gf)
-    gr = Grads()
-    gr.dL_dmeans3D, gr.dL_dmeans2D, gr.dL_dshs, gr.dL_dcolors = _ptr(d_means3D), _ptr(d_means2D), _ptr(d_sh), _ptr(d_colors)
-    gr.dL_dopacities, gr.dL_dscales, gr.dL_drotations, gr.dL_dcov3D = _ptr(d_opac), _ptr(d_scales), _ptr(d_rots), _ptr(d_cov)
-    gr.dL_dfeatures, gr.dL_dshs_language, gr.scratch = _ptr(d_feat), _ptr(d_shl), scratch.data_ptr()
-    if not camera:
-        check(lib.b200gs_backward(C.byref(v), C.byref(g), radii.data_ptr(), C.byref(ws), C.c_int64(capacity), C.byref(go),
-                                  C.byref(gr), _stream(dev)))
+    """The per-Gaussian tensors are the ones the forward read (_gaussians' output).  camera: () or the (shape, dtype) of
+    the viewmatrix, projmatrix and campos tensors whose gradients are wanted; the gradients are appended to the returned
+    tuple."""
+    inputs = dict(means3D=means3D, shs=sh, colors_precomp=colors_precomp, opacities=opacities, scales=scales, rotations=rotations,
+                  cov3D_precomp=cov3Ds_precomp, shs_language=shs_language, language_feature_precomp=language_feature_precomp,
+                  confidence=confidence)
+    P, dev = radii.shape[0], radii.device
+    grads = _grad_buffers(inputs, P, dev, extended, bool(camera))
+    if P > 0:
+        keep = []
+        g = _gaussians_struct(P, inputs)
+        v = _cached_view(rs, P, 0 if sh is None else int(sh.shape[1]), extended, keep)
+        go = GradOutputs()
+        gc = _f32c(g_color, "grad color")
+        gd, ga, gf = _f32c(g_depth, "grad depth"), _f32c(g_alpha, "grad alpha"), _f32c(g_feature, "grad feature")
+        go.dL_dcolor, go.dL_ddepth, go.dL_dalpha, go.dL_dfeature = _ptr(gc), _ptr(gd), _ptr(ga), _ptr(gf)
+        cg = _camera_struct(grads["camera"], grads["camera_scratch"]) if camera else None
+        _backward(v, g, radii, _workspace(geom, img, binning), capacity, go, _grads_struct(grads), cg, _stream(dev))
         del keep
-        return d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat
-    cam = got["cam"]
-    cg = CameraGrads()
-    cg.dL_dviewmatrix, cg.dL_dprojmatrix, cg.dL_dcampos = cam.data_ptr(), cam[16:].data_ptr(), cam[32:].data_ptr()
-    cg.scratch = got["cam_scratch"].data_ptr()
-    check(lib.b200gs_backward_camera(C.byref(v), C.byref(g), radii.data_ptr(), C.byref(ws), C.c_int64(capacity), C.byref(go),
-                                     C.byref(gr), C.byref(cg), _stream(dev)))
-    del keep
-    return (d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat) + _camera_grads(cam, camera)
+    elif camera:  # rasterize_points.cu:161: nothing is launched for an empty scene; its camera gradients are zeros
+        grads["camera"].zero_()
+    out = tuple([grads[k] for k in _GRADS])
+    return out + _camera_grads(grads["camera"], camera) if camera else out
 
 
 class _RasterizeGaussians(torch.autograd.Function):
@@ -321,28 +371,17 @@ class _RasterizeGaussians(torch.autograd.Function):
     def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
                 shs_language, language_feature_precomp, raster_settings, extended, *camera):
         """camera: () or (viewmatrix, projmatrix, campos) -- the settings' own tensors, passed again so that autograd
-        tracks them; backward then also returns their gradients."""
+        tracks them; backward then also returns their gradients.  What is saved for the backward are the per-Gaussian
+        tensors the kernels read (float32, contiguous copies of inputs that are not), so it reads what the forward read."""
         rs = raster_settings
-        confidence = getattr(rs, "confidence", None)
-        args = (rs, means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, shs_language,
-                language_feature_precomp, confidence, extended)
-        if rs.debug:
-            cpu_args = _cpu_deep_copy_tuple(args[1:])  # copy them before they can be corrupted
-            try:
-                res = _forward_impl(*args)
-            except Exception as ex:
-                torch.save(cpu_args, "snapshot_fw.dump")
-                print("\nAn error occured in forward. Please forward snapshot_fw.dump for debugging.")
-                raise ex
-        else:
-            res = _forward_impl(*args)
+        inputs, res = _with_snapshot(rs, "snapshot_fw.dump", "\nAn error occured in forward. Please forward snapshot_fw.dump for debugging.",
+                                     _forward, means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
+                                     shs_language, language_feature_precomp, getattr(rs, "confidence", None), extended)
         num_rendered, capacity, color, depth, alpha, feature, radii, geom, binning, img = res
         ctx.raster_settings = rs
         ctx.num_rendered, ctx.capacity, ctx.extended = num_rendered, capacity, extended
-        ctx.confidence = confidence
         ctx.camera = tuple((t.shape, t.dtype) for t in camera)
-        ctx.save_for_backward(colors_precomp, means3D, scales, rotations, cov3Ds_precomp, radii, sh, opacities,
-                              shs_language, language_feature_precomp, geom, binning, img)
+        ctx.save_for_backward(*inputs.values(), radii, geom, binning, img)
         ctx.mark_non_differentiable(radii)
         if extended:
             return color, depth, alpha, feature, radii
@@ -351,28 +390,12 @@ class _RasterizeGaussians(torch.autograd.Function):
     @staticmethod
     def backward(ctx, *grad_outs):
         rs = ctx.raster_settings
-        (colors_precomp, means3D, scales, rotations, cov3Ds_precomp, radii, sh, opacities, shs_language,
-         language_feature_precomp, geom, binning, img) = ctx.saved_tensors
-        if ctx.extended:
-            g_color, g_depth, g_alpha, g_feature = grad_outs[0], grad_outs[1], grad_outs[2], grad_outs[3]
-        else:
-            g_color, g_depth, g_alpha, g_feature = grad_outs[0], None, None, None
-        args = (rs, ctx.num_rendered, ctx.capacity, ctx.extended, means3D, sh, colors_precomp, opacities, scales,
-                rotations, cov3Ds_precomp, shs_language, language_feature_precomp, ctx.confidence, radii, geom,
-                binning, img, g_color, g_depth, g_alpha, g_feature, ctx.camera)
-        if rs.debug:
-            cpu_args = _cpu_deep_copy_tuple(args[1:])
-            try:
-                grads = _backward_impl(*args)
-            except Exception as ex:
-                torch.save(cpu_args, "snapshot_bw.dump")
-                print("\nAn error occured in backward. Writing snapshot_bw.dump for debugging.\n")
-                raise ex
-        else:
-            grads = _backward_impl(*args)
-        d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat = grads[:10]
+        g_out = grad_outs[:4] if ctx.extended else (grad_outs[0], None, None, None)
+        grads = _with_snapshot(rs, "snapshot_bw.dump", "\nAn error occured in backward. Writing snapshot_bw.dump for debugging.\n",
+                               _backward_impl, ctx.num_rendered, ctx.capacity, ctx.extended, *ctx.saved_tensors, *g_out,
+                               ctx.camera)
         # order of forward()'s inputs (reference order + the two SDP-GS tensors + settings + mode flag + camera tensors)
-        return (d_means3D, d_means2D, d_sh, d_colors, d_opac, d_scales, d_rots, d_cov, d_shl, d_feat, None, None) + tuple(grads[10:])
+        return grads[:10] + (None, None) + grads[10:]
 
 
 def rasterize_gaussians(means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
@@ -461,26 +484,10 @@ class RasterSession:
         self.dev = dev
         P = self.P = means3D.shape[0]
         H, W = int(rs.image_height), int(rs.image_width)
-        self._keep = []
-        f = lambda t, n: _f32c(t, n)
-        self.inputs = dict(means3D=f(means3D, "means3D"), opacities=f(opacities, "opacities"), shs=f(shs, "shs"),
-                           colors_precomp=f(colors_precomp, "colors_precomp"), scales=f(scales, "scales"),
-                           rotations=f(rotations, "rotations"), cov3D_precomp=f(cov3D_precomp, "cov3D_precomp"),
-                           shs_language=f(shs_language, "shs_language"),
-                           language_feature_precomp=f(language_feature_precomp, "language_feature_precomp"),
-                           confidence=f(getattr(rs, "confidence", None), "confidence"))
-        i = self.inputs
-        M = 0 if i["shs"] is None else int(i["shs"].shape[1])
-        g = self.g = Gaussians()
-        g.P = P
-        g.means3D, g.shs, g.colors_precomp, g.opacities = _ptr(i["means3D"]), _ptr(i["shs"]), _ptr(i["colors_precomp"]), _ptr(i["opacities"])
-        g.scales, g.rotations, g.cov3D_precomp = _ptr(i["scales"]), _ptr(i["rotations"]), _ptr(i["cov3D_precomp"])
-        g.language_feature_precomp, g.shs_language, g.confidence = _ptr(i["language_feature_precomp"]), _ptr(i["shs_language"]), _ptr(i["confidence"])
-        if live_count is not None:
-            if live_count.device != dev or live_count.numel() != 1 or live_count.dtype not in (torch.int32, torch.uint32):
-                raise RuntimeError("live_count must be a one-element int32/uint32 tensor on the session's device")
-            self._keep.append(live_count)
-            g.live_count = live_count.data_ptr()
+        self._keep = [] if live_count is None else [live_count]
+        self.inputs, self.g = _gaussians(means3D, shs, colors_precomp, opacities, scales, rotations, cov3D_precomp, shs_language,
+                                         language_feature_precomp, getattr(rs, "confidence", None), live_count)
+        M = 0 if self.inputs["shs"] is None else int(self.inputs["shs"].shape[1])
         self.v = _build_view(rs, P, M, self.extended, self._keep)
         f32 = dict(dtype=torch.float32, device=dev)
         self.color = torch.empty((3, H, W), **f32)
@@ -492,50 +499,26 @@ class RasterSession:
             self.depth, self.alpha, self.feature = torch.empty((1, H, W), **f32), torch.empty((1, H, W), **f32), torch.empty((3, H, W), **f32)
             o.depth, o.alpha, o.feature = self.depth.data_ptr(), self.alpha.data_ptr(), self.feature.data_ptr()
         u8 = dict(dtype=torch.uint8, device=dev)
-        self.geom = torch.empty((lib.b200gs_geom_bytes(P),), **u8)
-        self.img = torch.empty((lib.b200gs_image_bytes(W, H),), **u8)
+        gb, ib = _ws_bytes(P, W, H)
+        self.geom, self.img = torch.empty((gb,), **u8), torch.empty((ib,), **u8)
         self.binning = torch.empty((lib.b200gs_binning_bytes(self.capacity, W, H),), **u8)
-        ws = self.ws = Workspace()
-        ws.geom, ws.geom_bytes, ws.image, ws.image_bytes = self.geom.data_ptr(), self.geom.numel(), self.img.data_ptr(), self.img.numel()
-        ws.binning, ws.binning_bytes = self.binning.data_ptr(), self.binning.numel()
+        ws = self.ws = _workspace(self.geom, self.img, self.binning)
+        # persistent workspaces (b200gs_workspace_t.persistent): initialised once, left clean by the kernels, no memset per step
+        ws.persistent = 1
         self.graph = None
         self.with_backward = with_backward
         self.camera_grads, self.cg = None, None
-        if camera_grads and with_backward:
-            cam = torch.empty((64 + lib.b200gs_camera_scratch_bytes(P) // 4,), **f32)  # 35 outputs, then the scratch
-            self.camera_grads = dict(viewmatrix=cam[0:16].view(4, 4), projmatrix=cam[16:32].view(4, 4), campos=cam[32:35])
-            cg = self.cg = CameraGrads()
-            cg.dL_dviewmatrix, cg.dL_dprojmatrix, cg.dL_dcampos = cam.data_ptr(), cam[16:].data_ptr(), cam[32:].data_ptr()
-            cg.scratch = cam[64:].data_ptr()
-            self._keep.append(cam)
-        if not with_backward:
-            ws.persistent = 1
-            check(lib.b200gs_workspace_init(C.byref(ws), P, None, _stream(dev)))
         if with_backward:
-            go = grads_out or {}
-            has = lambda t: t is not None
-            mk = lambda name, shape, cond=True: (go.get(name) if go.get(name) is not None else torch.empty(shape, **f32)) if cond else None
-            self.grads = dict(
-                means3D=mk("means3D", (P, 3)), means2D=mk("means2D", (P, 3)), opacities=mk("opacities", (P, 1)),
-                shs=mk("shs", (P, M, 3), has(i["shs"])), colors_precomp=mk("colors_precomp", (P, 3), has(i["colors_precomp"])),
-                scales=mk("scales", (P, 3), has(i["scales"])), rotations=mk("rotations", (P, 4), has(i["rotations"])),
-                cov3D=mk("cov3D", (P, 6), has(i["cov3D_precomp"])),
-                features=mk("features", (P, 3), self.extended and has(i["language_feature_precomp"])),
-                shs_language=mk("shs_language", (P, 3), self.extended and has(i["shs_language"])))
-            for k, t in self.grads.items():
-                if t is not None and (not t.is_contiguous() or t.dtype != torch.float32):
-                    raise RuntimeError(f"grads_out[{k}] must be a contiguous float32 tensor")
-            self.scratch = torch.empty((lib.b200gs_scratch_bytes(P),), **u8)
-            gr = self.gr = Grads()
-            G = self.grads
-            gr.dL_dmeans3D, gr.dL_dmeans2D, gr.dL_dshs, gr.dL_dcolors = _ptr(G["means3D"]), _ptr(G["means2D"]), _ptr(G["shs"]), _ptr(G["colors_precomp"])
-            gr.dL_dopacities, gr.dL_dscales, gr.dL_drotations, gr.dL_dcov3D = _ptr(G["opacities"]), _ptr(G["scales"]), _ptr(G["rotations"]), _ptr(G["cov3D"])
-            gr.dL_dfeatures, gr.dL_dshs_language, gr.scratch = _ptr(G["features"]), _ptr(G["shs_language"]), self.scratch.data_ptr()
-            # persistent workspaces (b200gs_workspace_t.persistent): initialised once, left clean by the kernels, no memset per step
-            ws.persistent = 1
-            check(lib.b200gs_workspace_init(C.byref(ws), P, self.scratch.data_ptr(), _stream(dev)))
+            grads = _grad_buffers(self.inputs, P, dev, self.extended, camera_grads, grads_out)
+            self.grads = {k: grads[k] for k in _GRADS}
+            self.scratch = grads["scratch"]
+            gr = self.gr = _grads_struct(grads)
             if grad_scatter is not None:  # image-parallel training: parameter gradients are pushed to the owning ranks (parallel.FusedGradBuffer)
                 gr.scatter_bases, gr.scatter_shard_rows, gr.scatter_rank, gr.scatter_world = grad_scatter
+            if camera_grads:
+                cam = grads["camera"]
+                self.camera_grads = dict(viewmatrix=cam[0:16].view(4, 4), projmatrix=cam[16:32].view(4, 4), campos=cam[32:35])
+                self.cg = _camera_struct(cam, grads["camera_scratch"])
             self.cot = dict(color=torch.zeros((3, H, W), **f32))
             go_ = self.go = GradOutputs()
             go_.dL_dcolor = self.cot["color"].data_ptr()
@@ -543,19 +526,14 @@ class RasterSession:
                 self.cot.update(depth=torch.zeros((1, H, W), **f32), alpha=torch.zeros((1, H, W), **f32),
                                 feature=torch.zeros((3, H, W), **f32))
                 go_.dL_ddepth, go_.dL_dalpha, go_.dL_dfeature = self.cot["depth"].data_ptr(), self.cot["alpha"].data_ptr(), self.cot["feature"].data_ptr()
+        check(lib.b200gs_workspace_init(C.byref(ws), P, self.scratch.data_ptr() if with_backward else None, _stream(dev)))
 
     def forward(self):
         check(lib.b200gs_forward(C.byref(self.v), C.byref(self.g), C.byref(self.o), C.byref(self.ws),
                                  C.c_int64(self.capacity), _stream()))
 
     def backward(self):
-        if self.cg is not None:
-            check(lib.b200gs_backward_camera(C.byref(self.v), C.byref(self.g), self.radii.data_ptr(), C.byref(self.ws),
-                                             C.c_int64(self.capacity), C.byref(self.go), C.byref(self.gr), C.byref(self.cg),
-                                             _stream()))
-            return
-        check(lib.b200gs_backward(C.byref(self.v), C.byref(self.g), self.radii.data_ptr(), C.byref(self.ws),
-                                  C.c_int64(self.capacity), C.byref(self.go), C.byref(self.gr), _stream()))
+        _backward(self.v, self.g, self.radii, self.ws, self.capacity, self.go, self.gr, self.cg, _stream())
 
     def step(self):
         """forward, then backward with the cotangents currently stored in `self.cot` (fill them between the two

@@ -102,23 +102,23 @@ class GaussianTrainer:
         self.bucket = parallel.FusedGradBuffer(Pc, dev)
         self.g_means2D = torch.zeros((Pc, 3), dtype=torch.float32, device=dev)
         self._write_rows(raw, m, v, P_before=0)
-        C_ = self._cap["raw"]
-        grads_out = dict(means3D=self.bucket.segment("xyz"), shs=self.bucket.segment("shs"), opacities=self.bucket.segment("opacity"),
-                         scales=self.bucket.segment("scaling"), rotations=self.bucket.segment("rotation"),
-                         shs_language=self.bucket.segment("language_feature"), means2D=self.g_means2D)
         self._scatter = self.bucket.scatter_descriptor()
-        self.sessions = []
-        for cam in self.cameras:
-            s = rz.RasterSession(self.settings_fn(cam), means3D=C_["xyz"], opacities=self.act["opacity"],
-                                 shs=C_["shs"].view(Pc, 16, 3), scales=self.act["scaling"], rotations=self.act["rotation"],
-                                 shs_language=C_["feature"], extended=True, capacity=self.capacity, grads_out=grads_out,
-                                 grad_scatter=self.bucket.scatter_descriptor(), live_count=self.live)
-            self.sessions.append(s)
+        self.sessions = [self._session(cam, self.g_means2D) for cam in self.cameras]
         self.graphs = None
         self.pair_graphs = {}
         self.pseudo_sessions = []
         if getattr(self, "pseudo_cameras", None):
             self._build_pseudo_sessions()
+
+    def _session(self, cam, g_means2D):
+        """The RasterSession of one view over the capacity-sized buffers: parameter gradients go to the fused buffer,
+        the means2D gradient to `g_means2D`."""
+        Pc, C_, b = self.Pcap, self._cap["raw"], self.bucket
+        grads_out = dict(means3D=b.segment("xyz"), shs=b.segment("shs"), opacities=b.segment("opacity"), scales=b.segment("scaling"),
+                         rotations=b.segment("rotation"), shs_language=b.segment("language_feature"), means2D=g_means2D)
+        return rz.RasterSession(self.settings_fn(cam), means3D=C_["xyz"], opacities=self.act["opacity"], shs=C_["shs"].view(Pc, 16, 3),
+                                scales=self.act["scaling"], rotations=self.act["rotation"], shs_language=C_["feature"], extended=True,
+                                capacity=self.capacity, grads_out=grads_out, grad_scatter=b.scatter_descriptor(), live_count=self.live)
 
     def _write_rows(self, raw, m, v, P_before):
         """Install `raw` (and the moments; None = zeros) as rows [0, P) of the capacity-sized buffers, make rows [P, P_before)
@@ -160,17 +160,8 @@ class GaussianTrainer:
         self._build_pseudo_sessions()
 
     def _build_pseudo_sessions(self):
-        P = self.Pcap
-        C_ = self._cap["raw"]
-        self.g_means2D_pseudo = torch.zeros((P, 3), dtype=torch.float32, device=self.dev)  # not a densification input (train.py:220-221)
-        grads_out = dict(means3D=self.bucket.segment("xyz"), shs=self.bucket.segment("shs"), opacities=self.bucket.segment("opacity"),
-                         scales=self.bucket.segment("scaling"), rotations=self.bucket.segment("rotation"),
-                         shs_language=self.bucket.segment("language_feature"), means2D=self.g_means2D_pseudo)
-        self.pseudo_sessions = [rz.RasterSession(self.settings_fn(cam), means3D=C_["xyz"], opacities=self.act["opacity"],
-                                                 shs=C_["shs"].view(P, 16, 3), scales=self.act["scaling"], rotations=self.act["rotation"],
-                                                 shs_language=C_["feature"], extended=True, capacity=self.capacity, grads_out=grads_out,
-                                                 grad_scatter=self.bucket.scatter_descriptor(), live_count=self.live)
-                                for cam in self.pseudo_cameras]
+        self.g_means2D_pseudo = torch.zeros((self.Pcap, 3), dtype=torch.float32, device=self.dev)  # not a densification input (train.py:220-221)
+        self.pseudo_sessions = [self._session(cam, self.g_means2D_pseudo) for cam in self.pseudo_cameras]
         self.pair_graphs = {}
 
     def set_pseudo_weight(self, w):

@@ -45,13 +45,10 @@ def _stream():
 
 def _cam_struct(P):
     """NaN-filled camera outputs and a NaN-filled scratch (the partials are assigned, never accumulated)."""
-    L = _lib()
+    from b200gs.rasterizer import _camera_struct
     out = torch.full((35,), float("nan"), device="cuda")
-    scratch = torch.full((int(L.lib.b200gs_camera_scratch_bytes(P)) // 4,), float("nan"), device="cuda")
-    cg = L.CameraGrads()
-    cg.dL_dviewmatrix, cg.dL_dprojmatrix, cg.dL_dcampos = out.data_ptr(), out[16:].data_ptr(), out[32:].data_ptr()
-    cg.scratch = scratch.data_ptr()
-    return out, scratch, cg
+    scratch = torch.full((int(_lib().lib.b200gs_camera_scratch_bytes(P)) // 4,), float("nan"), device="cuda")
+    return out, scratch, _camera_struct(out, scratch)
 
 
 def _backward_camera(s, cg):
