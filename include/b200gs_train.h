@@ -108,9 +108,19 @@ int b200gs_depth_pearson_loss_pseudo(const float* depth, const float* depth_ref,
  * its simple_knn fork (`dist, nearest_indices = distCUDA2(xyz)`, scene/gaussian_model.py:513-516; the extension is not
  * vendored under /root/reference, SURVEY.md F5).  mean_dist2[i] = mean of the three squared distances (simple_knn's
  * definition), indices[i] = the neighbours in order of increasing distance (ties: lower index first).
- * Tiled brute force, O(P^2 / 1024) shared-memory passes: meant for the few-shot regime (P ~ 1e5) in which proximity()
- * runs (iteration < 2000). */
+ * Tiled brute force, O(P^2 / 1024) shared-memory passes: the faster choice for small clouds, and the reference that
+ * b200gs_knn3_tree is tested against.  Points with a non-finite coordinate are nobody's neighbour; a point with fewer than
+ * three finite neighbours within squared distance 3e38 gets index -1 and distance 3e38 in the missing places. */
 int b200gs_knn3(int32_t P, const float* xyz, float* mean_dist2, int32_t* indices, void* stream);
+
+/* Bytes of device scratch b200gs_knn3_tree needs for P points (0 when P is out of range). */
+size_t b200gs_knn3_scratch_bytes(int32_t P);
+/* Same outputs, bit for bit, as b200gs_knn3 on every input; O(P log P) work (Morton-ordered implicit box hierarchy,
+ * knn.cu); no host synchronisation, so the call can be captured in a CUDA graph.
+ * 4 <= P < 2^30 (the onesweep look-back counters); scratch needs no initialisation.  B200GS_E_ARG, with nothing launched,
+ * when P is out of range, a pointer is NULL or scratch_bytes < b200gs_knn3_scratch_bytes(P). */
+int b200gs_knn3_tree(int32_t P, const float* xyz, float* mean_dist2, int32_t* indices,
+                     void* scratch, size_t scratch_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -85,7 +85,8 @@ class ParamState(C.Structure):  # b200gs_param_state_t
 
 
 TRAIN_EXPORTS = ["b200gs_param_step", "b200gs_photometric_loss", "b200gs_photometric_scratch_bytes",
-                 "b200gs_depth_pearson_loss", "b200gs_hparams_advance", "b200gs_loss_accum_doubles", "b200gs_knn3", "b200gs_depth_pearson_loss_pseudo", "b200gs_train_abi_sizes"]
+                 "b200gs_depth_pearson_loss", "b200gs_hparams_advance", "b200gs_loss_accum_doubles", "b200gs_knn3", "b200gs_depth_pearson_loss_pseudo", "b200gs_train_abi_sizes",
+                 "b200gs_knn3_scratch_bytes", "b200gs_knn3_tree"]
 COLLECTIVE_EXPORTS = ["b200gs_allreduce_sum_f32", "b200gs_allreduce_flag_words", "b200gs_gather_reduce_f32"]
 
 EXPORTS = [
@@ -146,6 +147,9 @@ def _load():
     lib.b200gs_depth_pearson_loss_pseudo.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
                                                      C.c_void_p, C.c_void_p, C.c_void_p]
     lib.b200gs_knn3.argtypes = [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.b200gs_knn3_scratch_bytes.argtypes = [C.c_int32]
+    lib.b200gs_knn3_scratch_bytes.restype = C.c_size_t
+    lib.b200gs_knn3_tree.argtypes = [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
     lib.b200gs_hparams_advance.argtypes = [C.c_void_p, C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p]
     lib.b200gs_allreduce_flag_words.argtypes = [C.c_int32]
     lib.b200gs_allreduce_flag_words.restype = C.c_size_t

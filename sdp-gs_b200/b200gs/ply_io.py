@@ -9,6 +9,9 @@ for an all-'f4' structured array (plyfile is not in this image; the format is wr
 (`features.transpose(1, 2).flatten(start_dim=1)`): f_rest_{c*15 + k} = shs[:, 1 + k, c].
 Arrays use this repo's trainer layout: xyz [P,3], shs [P,16,3], opacity [P,1], scaling [P,3], rotation [P,4],
 feature [P,3] or None.
+
+`load_point_cloud` reads the input point cloud of scene initialisation (fetchPly, scene/dataset_readers.py): a vertex PLY
+with x y z red green blue, such as COLMAP's points3D.ply.
 """
 from __future__ import annotations
 
@@ -114,3 +117,14 @@ def load_ply(path, max_sh_degree=3):
     feat_names = sorted((n for n in names if n.startswith("languagefeature_")), key=lambda x: int(x.split("_")[-1]))
     feature = np.stack([v[n] for n in feat_names], axis=1).astype(np.float32) if feat_names else None
     return dict(xyz=xyz, shs=np.ascontiguousarray(shs), opacity=opacity, scaling=scaling, rotation=rotation, feature=feature)
+
+
+def load_point_cloud(path):
+    """(xyz f32[P,3], rgb f32[P,3] in [0, 1]) of a vertex PLY with x, y, z, red, green, blue; `uchar` colours are divided
+    by 255 as fetchPly does."""
+    v = read_vertex_table(path)
+    xyz = np.stack((v["x"], v["y"], v["z"]), axis=1).astype(np.float32)
+    rgb = np.stack((v["red"], v["green"], v["blue"]), axis=1)
+    if rgb.dtype == np.uint8:
+        rgb = rgb / 255.0
+    return xyz, rgb.astype(np.float32)

@@ -24,12 +24,36 @@ import math
 import numpy as np
 import torch
 
+from . import knn
 from . import parallel
 from . import rasterizer as rz
 from ._lib import HParams, ParamState, check, lib
 
 from .schedule import DEFAULTS, expon_lr  # noqa: E402,F401  (pure Python: importable without the native library)
 from .densify_logic import build_rotation, densify_rows  # noqa: E402  (pure torch)
+
+
+def params_from_point_cloud(xyz, rgb, device, sh_degree=3):
+    """The raw parameters GaussianTrainer starts from for an input point cloud (create_from_pcd,
+    scene/gaussian_model.py:186-212): f_dc = (rgb - 0.5) / C0 and the rest of the SH zero, opacity logit(0.1), scaling
+    log(sqrt(max(mean squared distance to the 3 nearest neighbours, 1e-7))) on all three axes, rotation (1, 0, 0, 0),
+    feature zero.  xyz, rgb: [P,3] arrays (rgb in [0, 1]); returns float32 numpy arrays keyed by GaussianTrainer's
+    argument names."""
+    dev = torch.device(device)
+    x = torch.as_tensor(np.asarray(xyz), dtype=torch.float32, device=dev).reshape(-1, 3)
+    c = torch.as_tensor(np.asarray(rgb), dtype=torch.float32, device=dev).reshape(-1, 3)
+    P = x.shape[0]
+    shs = torch.zeros((P, (sh_degree + 1) ** 2, 3), dtype=torch.float32, device=dev)
+    shs[:, 0] = (c - 0.5) / 0.28209479177387814
+    dist2 = torch.clamp_min(knn.knn3(x)[0], 0.0000001)
+    scaling = torch.log(torch.sqrt(dist2))[..., None].repeat(1, 3)
+    rotation = torch.zeros((P, 4), dtype=torch.float32, device=dev)
+    rotation[:, 0] = 1
+    o = 0.1 * torch.ones((P, 1), dtype=torch.float32, device=dev)
+    opacity = torch.log(o / (1 - o))
+    out = dict(xyz=x, shs=shs, opacity_raw=opacity, scaling_raw=scaling, rotation_raw=rotation,
+               feature=torch.zeros((P, 3), dtype=torch.float32, device=dev))
+    return {k: v.cpu().numpy() for k, v in out.items()}
 
 
 class GaussianTrainer:
@@ -413,12 +437,7 @@ class GaussianTrainer:
 
     def knn3(self, xyz):
         """(mean squared distance to the 3 nearest neighbours [P], their indices [P,3]) -- distCUDA2 of the SDP-GS simple_knn fork."""
-        xyz = xyz.detach().contiguous().float()
-        P = xyz.shape[0]
-        dist = torch.empty((P,), dtype=torch.float32, device=xyz.device)
-        idx = torch.empty((P, 3), dtype=torch.int32, device=xyz.device)
-        check(lib.b200gs_knn3(P, xyz.data_ptr(), dist.data_ptr(), idx.data_ptr(), rz._stream()))
-        return dist, idx
+        return knn.knn3(xyz)
 
     def densify_and_prune(self, max_grad, min_opacity, extent, max_screen_size, iteration=None, percent_dense=0.01,
                           prune_from_iter=500, N=2, generator=None, recapture=True, proximity_until_iter=2000):

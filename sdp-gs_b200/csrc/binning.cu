@@ -566,11 +566,10 @@ void launch_finalize_header(const RasterPlan& pl, cudaStream_t stream) {
 	launch(PDL_EMIT, finalize_header_kernel, dim3(1), dim3(1), 0, stream, pl.gs.hdr, (long long)pl.capacity);
 }
 
-// stable LSD radix sort of (u32 key, u32 value) pairs on key bits [0, end_bit); n is read from *n_dev (clamped to n_max) when
-// n_dev != nullptr, else n = n_max.  The result is in (key_a, val_a) after an even number of passes, else in (key_b, val_b).
-static void launch_radix_sort(uint32_t* key_a, uint32_t* key_b, uint32_t* val_a, uint32_t* val_b, int64_t n_max,
-                              const unsigned long long* n_dev, int end_bit, uint32_t* hist /*[passes][256]*/, uint32_t* lookback,
-                              unsigned int* tickets, unsigned int* barrier /*zero on entry*/, cudaStream_t stream) {
+// (declared in common.cuh)
+void launch_radix_sort(uint32_t* key_a, uint32_t* key_b, uint32_t* val_a, uint32_t* val_b, int64_t n_max,
+                       const unsigned long long* n_dev, int end_bit, uint32_t* hist /*[passes][256]*/, uint32_t* lookback,
+                       unsigned int* tickets, unsigned int* barrier /*zero on entry*/, cudaStream_t stream) {
 	if (n_max <= 0 || end_bit <= 0) return;
 	const int passes = (end_bit + 7) / 8;
 	const int items = sort_items_for(n_max);

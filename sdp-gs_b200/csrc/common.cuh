@@ -148,6 +148,13 @@ void launch_tile_sort(const RasterPlan& pl, cudaStream_t stream);
 void launch_tile_ranges(const RasterPlan& pl, int64_t n_max /* 0: nothing was emitted */, cudaStream_t stream);
 void launch_finalize_header(const RasterPlan& pl, cudaStream_t stream);
 void launch_debug_keys(const RasterPlan& pl, uint64_t* keys_out, int64_t L, cudaStream_t stream);
+// Stable LSD radix sort of (u32 key, u32 value) pairs on key bits [0, end_bit) (binning.cu); n is read from *n_dev (clamped to
+// n_max) when n_dev != nullptr, else n = n_max.  The result is in (key_a, val_a) after an even number of passes, else in
+// (key_b, val_b).  hist[p][256]: the digit counts of pass p, produced by the kernel that wrote the keys.  lookback
+// ([passes][sort_tiles_for(n_max)][256] words), tickets[passes] and *barrier must be zero on entry.
+void launch_radix_sort(uint32_t* key_a, uint32_t* key_b, uint32_t* val_a, uint32_t* val_b, int64_t n_max,
+                       const unsigned long long* n_dev, int end_bit, uint32_t* hist, uint32_t* lookback,
+                       unsigned int* tickets, unsigned int* barrier, cudaStream_t stream);
 
 void launch_blend_forward(const RasterPlan& pl, const b200gs_outputs_t& out, cudaStream_t stream);  // also writes bs.surv_bits
 void launch_blend_backward(const RasterPlan& pl, const b200gs_grad_outputs_t& gout, float* grec, cudaStream_t stream);

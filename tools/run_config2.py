@@ -40,7 +40,6 @@ A = ap.parse_args()
 dev = torch.device("cuda", 0)
 torch.cuda.set_device(0)
 W, H = 504, 378
-SH_C0 = 0.28209479177387814
 
 # ---- schedule (run_llff_mvs.sh:9-22 over arguments/__init__.py:74-125)
 HP = dict(DEFAULTS)
@@ -95,17 +94,8 @@ with torch.no_grad():
 # ---- the initial cloud (scene/gaussian_model.py:186-212 on random points, scene/dataset_readers.py:553-555)
 rng = np.random.default_rng(77 + A.seed)
 xyz0 = (rng.uniform(-1.0, 1.0, size=(A.P0, 3)) * 1.3 * gt.extent).astype(np.float32)
-shs0 = np.zeros((A.P0, 16, 3), np.float32)
-shs0[:, 0] = (rng.uniform(0, 1, size=(A.P0, 3)) - 0.5) / SH_C0
-from b200gs._lib import lib, check  # noqa: E402
-from b200gs import rasterizer as rz  # noqa: E402
-_x = t(xyz0)
-_d = torch.empty((A.P0,), device=dev); _i = torch.empty((A.P0, 3), dtype=torch.int32, device=dev)
-check(lib.b200gs_knn3(A.P0, _x.data_ptr(), _d.data_ptr(), _i.data_ptr(), rz._stream()))
-dist2 = torch.clamp_min(_d, 1e-7).cpu().numpy()
-raw0 = dict(xyz=xyz0, shs=shs0, opacity_raw=np.full((A.P0, 1), np.log(0.1 / 0.9), np.float32),
-            scaling_raw=np.repeat(np.log(np.sqrt(dist2))[:, None], 3, axis=1).astype(np.float32),
-            rotation_raw=np.tile(np.array([[1, 0, 0, 0]], np.float32), (A.P0, 1)), feature=np.zeros((A.P0, 3), np.float32))
+from b200gs.trainer import params_from_point_cloud  # noqa: E402
+raw0 = params_from_point_cloud(xyz0, rng.uniform(0, 1, size=(A.P0, 3)), dev)
 
 
 def sequence(seed):
